@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...   the reference's own C receiver on host cores
+  python bench.py ... --dump-outputs DIR                    also writes rank 0's receiver state after the last timed step
+                                                            (seeded inputs: two builds can be compared array for array)
 
 Metric (BASELINE.json): tracking channel*Msamples/s = streams x 12 channels x complex samples / time,
 closed loop (correlator + channel logic) included.  Workload: BASELINE config 5 -- 64 independent
@@ -58,6 +60,8 @@ def parse():
     ap.add_argument("--no-also", action="store_true", help="skip the extra tracking shapes (C2 single stream, 64 streams on one GPU)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="length of the stream sample the CPU baseline processes")
     ap.add_argument("--ref-sample-seconds", type=float, default=1.0, help="per-stream sample of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the receivers' state after the last timed step as DIR/rx_<field>.npy (float64), to compare two builds")
     return ap.parse_args()
 
 
@@ -148,6 +152,28 @@ def profile_constant(key: str):
         return None
     with open(p) as f:
         return json.load(f).get(key)
+
+
+def dump_rx(out_dir: str, rx) -> None:
+    """Every field of the receivers' state (what gnssb200_download_rx returns to the caller) as out_dir/rx_<field>.npy
+    in float64, leading axis = stream.  A 64-bit integer field gets a last axis of two, (high 32 bits, low 32 bits), so
+    that every value stays exact."""
+    os.makedirs(out_dir, exist_ok=True)
+    a = np.ctypeslib.as_array(rx)
+
+    def walk(arr, prefix):
+        for name in arr.dtype.names:
+            if name == "pad_":
+                continue
+            v = arr[name]
+            if v.dtype.names:
+                walk(v, f"{prefix}{name}_")
+                continue
+            if v.dtype.itemsize == 8 and v.dtype.kind in "iu":
+                v = np.stack([v >> 32, v & 0xFFFFFFFF], axis=-1)
+            np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), v.astype(np.float64))
+
+    walk(a, "rx_")
 
 
 # --------------------------------------------------------------------------------------------------
@@ -310,6 +336,8 @@ def run_ours(args):
     value = total_chan_samples * args.steps / (t_ms_max * 1e-3) / 1e6
     eng.download()
     states = [int(eng.rx[s].chan[ch].state) for s in range(S) for ch in range(12)]
+    if args.dump_outputs and rank == 0:
+        dump_rx(args.dump_outputs, eng.rx)
 
     # ---- end to end through the host-buffer C ABI call ----
     h_if = torch.empty((S, stream_bytes), dtype=torch.uint8).pin_memory()

@@ -23,8 +23,6 @@ def oracle_lib():
 @pytest.fixture(scope="session")
 def track_record():
     """~1.75 s GPS record, three satellites in Doppler bins +1/-1/+1 (seed 2002-like)."""
-    import numpy as np
-
     from gnss_sdr_ru_b200.synth import Sat, make_record
 
     nblk = 3400
@@ -33,10 +31,5 @@ def track_record():
         Sat(prn=9, doppler_hz=-900, cn0_dbhz=47, code_phase_chips=980.0, data_seed=6),
         Sat(prn=32, doppler_hz=1000, cn0_dbhz=49, code_phase_chips=1010.0, data_seed=7),
     ]
-    cache = f"/tmp/gnssb200_track_record_{nblk}.npy"
-    if os.path.exists(cache):
-        rec = np.load(cache)
-    else:
-        rec = make_record(sats, 8192 * nblk, seed=2002)
-        np.save(cache, rec)
-    return rec, nblk
+    # generated in every session: a file shared between runs could come from another version of synth.py
+    return make_record(sats, 8192 * nblk, seed=2002), nblk
