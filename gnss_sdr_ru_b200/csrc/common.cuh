@@ -20,6 +20,11 @@ __host__ __device__ __forceinline__ long long code_table_base(int prn_reg) {
   if (prn_reg == GNSSB200_PRN_GLONASS) return (long long)GLO_ROW * HALF_CHIPS;
   return (prn_reg >= 0 && prn_reg <= 33) ? (long long)prn_reg * HALF_CHIPS : -1;
 }
+// End of what a channel may read: a GPS row spills over into the rows after it like the reference's flat reads, but
+// only up to the end of row 33 (the reference has 33 rows; reads past the zero row 33 give 0, never the ST code of row
+// 35).  Only the GLONASS row reaches into rows 35 and 36.
+#define GPS_TABLE_END (34 * HALF_CHIPS)
+__host__ __device__ __forceinline__ long long code_row_end(int prn_reg) { return prn_reg == GNSSB200_PRN_GLONASS ? TABLE_ENTRIES : GPS_TABLE_END; }
 __host__ __device__ __forceinline__ int code_period(int prn_reg) { return prn_reg == GNSSB200_PRN_GLONASS ? GLO_HALF_CHIPS : HALF_CHIPS; }
 __host__ __device__ __forceinline__ bool code_has_fast_row(int prn_reg) { return (prn_reg >= 1 && prn_reg <= 32) || prn_reg == GNSSB200_PRN_GLONASS; }
 

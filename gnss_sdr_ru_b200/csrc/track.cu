@@ -250,7 +250,7 @@ int track_launch(gnssb200_handle *h, int first_stream, int n_streams, const void
     if (h->device < 0 || h->device >= 64 || !aws[h->device]) {
       CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<2, GNSSB200_FMT_INT8_IQ, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_I8));
       CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<3, GNSSB200_FMT_INT8_IQ, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_I8));
-      CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<5, GNSSB200_FMT_INT8_IQ, 96, 11>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_I8));
+      CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<5, GNSSB200_FMT_INT8_IQ, 128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_I8));
       CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<2, GNSSB200_FMT_PACKED2, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_PK));
       CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<3, GNSSB200_FMT_PACKED2, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_PK));
       CUDA_TRY(cudaFuncSetAttribute(track_ws_kernel<1, GNSSB200_FMT_PACKED2, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, DSM_PK));
@@ -325,8 +325,12 @@ int track_launch(gnssb200_handle *h, int first_stream, int n_streams, const void
       if (form >= 3) seg = true;  // forced: out-of-range blocks take the per-sample form inside the kernel
     }
     const size_t dyn_seg = dyn + 2048;  // slack to start the mixer table on a 2048-byte boundary
-    if (fmt == GNSSB200_FMT_INT8_IQ && seg && (form == 0 || form == 3))  // segment form on int8 I,Q samples; 224 bytes of read-ahead behind the second tile
-      track_ws_kernel<5, GNSSB200_FMT_INT8_IQ, 96, 11><<<items, 128, dyn + 256, st>>>(a, tile_bytes);
+    // segment form on int8 I,Q samples; 224 bytes of read-ahead behind the second tile.  Eight segments per thread: a
+    // thread sums up to 8 x 8 samples of up to 384 per 16-bit lane before it unpacks them (24576 <= 32767 for any int8
+    // input; eleven segments could reach 33792 and carry into the other lane).  127 x 8 = 1016 of the ~1048 segments
+    // of an 8192-sample block are owned, the rest is the tail.
+    if (fmt == GNSSB200_FMT_INT8_IQ && seg && (form == 0 || form == 3))
+      track_ws_kernel<5, GNSSB200_FMT_INT8_IQ, 128, 8><<<items, 160, dyn + 256, st>>>(a, tile_bytes);
     else if (fmt == GNSSB200_FMT_INT8_IQ && per_sm >= 3)
       track_ws_kernel<3, GNSSB200_FMT_INT8_IQ, 256><<<items, 288, dyn, st>>>(a, tile_bytes);
     else if (fmt == GNSSB200_FMT_INT8_IQ)

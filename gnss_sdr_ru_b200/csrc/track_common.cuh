@@ -25,6 +25,10 @@ __device__ unsigned g_track_check_fail[8];
 // slew) before the dump and below the half chips one block spans (~1050) after it, each plus the few entries
 // a chunk reads ahead; larger slews take the serial path.
 #define SMEM_TBL 2304
+// The copies of that window (track_ws_kernel, track_loop_kernel) are bounded by TABLE_ENTRIES only: for the fast rows
+// (PRN 1..32, GLONASS) the window never reaches a row the register may not read (serial_block, which follows any slew,
+// bounds every read by code_row_end).
+static_assert(32 * HALF_CHIPS + SMEM_TBL <= GPS_TABLE_END, "the shared code-table window of PRN 32 reaches past row 33");
 
 struct StepParams {
   uint32_t cph0, kph0, cinc, kinc;
@@ -477,12 +481,12 @@ __device__ __noinline__ void serial_block(ChanShared &cs, const StepParams &sp, 
                                           const uint8_t *blk) {
   gnssb200_corr &g = cs.g;
   ChRegs &r = cs.r;
-  const long long row = code_table_base(r.w_prn);
+  const long long row = code_table_base(r.w_prn), row_end = code_row_end(r.w_prn);
   const int dump_at = r.w_slew + code_period(r.w_prn);
   uint16_t hc = (uint16_t)g.half_chip;
   auto bits_at = [&](uint16_t hh) -> uint32_t {
     long long f = row + hh;
-    return (row >= 0 && f < TABLE_ENTRIES) ? code_table[f] : 0u;
+    return (row >= 0 && f < row_end) ? code_table[f] : 0u;
   };
   uint32_t t = bits_at(hc);
   int cE = sext8(t, 0), cP = sext8(t, 1), cL = sext8(t, 2);

@@ -67,7 +67,8 @@ __device__ __forceinline__ uint32_t seg_start(uint32_t m, double nk05 /* -kph0 -
 // H whole segments starting at sample s: q = bit address of the sample's 4-bit code in shared memory (8 * byte
 // address of the tile + 4*s), cph / ks = carrier / code NCO phase at s (ks < kinc), hp = shared-memory byte address
 // of the first segment's code-table entry (consecutive entries follow), nvalid = segments that count.
-// Sums come back as two 16-bit lanes (ival + 65536*qval), |lane| <= 8*H*9.
+// Sums come back as two 16-bit lanes (ival + 65536*qval), |lane| <= 8*H*9 for packed samples (|ival|, |qval| <= 9
+// per sample); unpack_lanes is exact while |lane| <= 32767 (tests/test_track_bounds.py checks every launched H).
 struct SegBounds {  // shared-memory windows the loop may touch (TRACK_CHECK builds)
   uint32_t tile_lo, tile_hi, bits_lo, bits_hi, vlut_lo, vlut_hi;
 };
@@ -172,15 +173,19 @@ __device__ __forceinline__ void correlate_segments(uint32_t q, uint32_t cph, uin
   accL = aL;
 }
 
-// The segment loop on int8 I,Q samples (the reference's own file format, 2 bytes per sample, any int8 value): the
+// The segment loop on int8 I,Q samples (the reference's own file format, 2 bytes per sample): the
 // mixer is the reference's two multiplications per output (correlator.c:214-215) with the LO pair
 // (ival + 65536*qval coefficients of I and Q, fill_lo_lut) read from an 8-entry shared table -- one LDS.64, two
 // PRMT sign extensions, two IMADs per sample -- and the three code multiplications once per half chip as above.
 // q = bit address of the sample's I byte (8 * tile address + 16*s): a segment's 16 bytes come from five aligned words.
+// One int8 sample adds up to 2*128 + 1*128 = 384 to a lane (|lo_i| + |lo_q| = 3), so the run is exact for any int8
+// input only while 8*H*384 <= 32767, i.e. H <= 10 (a full-scale run of 11 segments reaches 33792 and carries into the
+// other lane).
 template <int H>
 __device__ __forceinline__ void correlate_segments_i8(uint32_t q, uint32_t cph, uint32_t ks, const uint32_t cinc, const uint32_t kinc,
                                                       const uint32_t k7, const uint32_t hp, const int nvalid, const uint32_t lut_addr,
                                                       const PipeK K, int &accE, int &accP, int &accL, const SegBounds bnd) {
+  static_assert(8 * H * 384 <= 32767, "int8 segment run: a 16-bit lane of the packed sums can overflow");
   int aE = 0, aP = 0, aL = 0;
   TCHECK(0, ks < kinc || nvalid == 0);
   TCHECK(1, hp >= bnd.bits_lo && hp + 4u * (H + 1) <= bnd.bits_hi + 4u);

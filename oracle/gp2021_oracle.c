@@ -16,7 +16,9 @@
  *
  * One documented deviation, shared with libosgnss_ref34.so: reads past a PRN's 2046-entry row
  * continue into the next row as in the reference (flat indexing), and past row 33 return 0
- * (the reference's arrays are [33][2046]; reading further is undefined there).
+ * (the reference's arrays are [33][2046]; reading further is undefined there).  The GLONASS
+ * ST-code row (35) lies behind that end: only GNSSB200_PRN_GLONASS reads it, a GPS row never
+ * spills into it.
  */
 #include <math.h>
 #include <stdint.h>
@@ -87,22 +89,24 @@ static long code_table_base(int prn_reg) {
   return (prn_reg >= 0 && prn_reg <= 33) ? (long)prn_reg * HALF_CHIPS : -1;
 }
 static int code_period(int prn_reg) { return prn_reg == GNSSB200_PRN_GLONASS ? GLO_HALF_CHIPS : HALF_CHIPS; }
+/* first flat index a PRN register may no longer read: a GPS row spills over up to the end of row 33 (34 rows, as in
+   libosgnss_ref34.so), the GLONASS row up to the end of the table */
+static long code_row_end(int prn_reg) { return prn_reg == GNSSB200_PRN_GLONASS ? (long)TABLE_ROWS * HALF_CHIPS : 34L * HALF_CHIPS; }
 static long long carrier_ref_of(const gnssb200_chan *k, const gnssb200_cfg *c) { return k->system ? c->glonass_carrier_ref : c->gps_carrier_ref; }
 static long long code_ref_of(const gnssb200_chan *k, const gnssb200_cfg *c) { return k->system ? c->glonass_code_ref : c->gps_code_ref; }
 
 /* E/P/L entry (which = 0 early, 1 prompt, 2 late) of half chip h for a PRN register value: for tests of the tables */
+/* flat table read with the reference's row spill-over; at or past `end` (code_row_end) -> 0 */
+static inline int tab_at(const int8_t *t, long flat, long end) {
+  return (flat >= 0 && flat < end) ? t[flat] : 0;
+}
+
 int orc_code_bit(int which, int prn_reg, int h) {
   build_tables();
   const long base = code_table_base(prn_reg);
   if (base < 0) return 0;
   const int8_t *t = which == 0 ? tab_early : (which == 1 ? tab_prompt : tab_late);
-  const long f = base + h;
-  return (f >= 0 && f < (long)TABLE_ROWS * HALF_CHIPS) ? t[f] : 0;
-}
-
-/* flat table read with the reference's row spill-over; outside the 34 rows -> 0 */
-static inline int tab_at(const int8_t *t, long flat) {
-  return (flat >= 0 && flat < (long)TABLE_ROWS * HALF_CHIPS) ? t[flat] : 0;
+  return tab_at(t, base + h, code_row_end(prn_reg));
 }
 
 /* 8-phase LO of the carrier mixer, OSG/correlator/correlator.c:203-204 (= NAM/rtl/carrier_nco.v:21-25) */
@@ -113,13 +117,9 @@ void orc_lo_table(int phase, int out[2]) {
   out[1] = lo_q[phase & 7];
 }
 
-/* expose for tests: E/P/L at (prn, h) */
+/* expose for tests: E/P/L at (PRN register, h) */
 void orc_code_bits(int prn, int h, int out[3]) {
-  build_tables();
-  long f = (long)prn * HALF_CHIPS + h;
-  out[0] = tab_at(tab_early, f);
-  out[1] = tab_at(tab_prompt, f);
-  out[2] = tab_at(tab_late, f);
+  for (int w = 0; w < 3; w++) out[w] = orc_code_bit(w, prn, h);
 }
 
 /* ------------------------------------------------------------------------------------------- */
@@ -265,8 +265,10 @@ void orc_sim_gp2021(gnssb200_rx *rx, const gnssb200_cfg *c, const int8_t *IF, lo
     const uint32_t cinc = (uint32_t)((W[base + 3] << 16) + W[base + 4]); /* :187 */
     const uint32_t kinc = (uint32_t)((W[base + 5] << 16) + W[base + 6]) << 1; /* :189,:245 */
     const long row = code_table_base(W[base]) >= 0 ? code_table_base(W[base]) : (long)TABLE_ROWS * HALF_CHIPS; /* no code: reads give 0 */
+    const long row_end = code_row_end(W[base]);
     uint16_t hc = (uint16_t)g->half_chip;
-    int bp = tab_at(tab_prompt, row + hc), bl = tab_at(tab_late, row + hc), be = tab_at(tab_early, row + hc); /* :196-198 */
+    int bp = tab_at(tab_prompt, row + hc, row_end), bl = tab_at(tab_late, row + hc, row_end),
+        be = tab_at(tab_early, row + hc, row_end); /* :196-198 */
     const int8_t *p = IF;
 
     for (long i = 0; i < nsamp; i++) {
@@ -299,9 +301,9 @@ void orc_sim_gp2021(gnssb200_rx *rx, const gnssb200_cfg *c, const int8_t *IF, lo
         g->code_phase += kinc;
         if (g->code_phase < before) {
           hc++;
-          bp = tab_at(tab_prompt, row + hc);
-          bl = tab_at(tab_late, row + hc);
-          be = tab_at(tab_early, row + hc);
+          bp = tab_at(tab_prompt, row + hc, row_end);
+          bl = tab_at(tab_late, row + hc, row_end);
+          be = tab_at(tab_early, row + hc, row_end);
           if (hc >= dump_at) {
             for (int a = 0; a < 6; a++) {
               R[base + 0x84 + a] = g->acc[a];
