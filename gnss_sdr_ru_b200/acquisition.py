@@ -63,6 +63,20 @@ class Settings:
         return c
 
 
+def _results(res) -> dict:
+    """acqResults fields of a gnssb200_acq_result array (the form acquisition() returns)."""
+    return dict(
+        carrFreq=np.array([r.carrFreq for r in res]),
+        codePhase=np.array([r.codePhase for r in res]),
+        peakMetric=np.array([r.peakMetric for r in res]),
+        freqChannel=np.array([r.sv for r in res]),
+        bin=np.array([r.bin for r in res]),
+        codePhaseRaw=np.array([r.codePhaseRaw for r in res]),
+        peak=np.array([r.peak for r in res]),
+        second=np.array([r.second for r in res]),
+    )
+
+
 class AcquisitionEngine:
     def __init__(self, device: int = 0, handle=None):
         self.L = lib()
@@ -109,16 +123,7 @@ class AcquisitionEngine:
         rows = np.zeros((n_sv, nb), dtype=abi.ACQ_ROW_DTYPE)
         check(self.L.gnssb200_acq_pcps_host(self.h, C.byref(c), buf.ctypes.data, fmt, n_samples, res, rows.ctypes.data),
               "gnssb200_acq_pcps_host")
-        out = dict(
-            carrFreq=np.array([r.carrFreq for r in res]),
-            codePhase=np.array([r.codePhase for r in res]),
-            peakMetric=np.array([r.peakMetric for r in res]),
-            freqChannel=np.array([r.sv for r in res]),
-            bin=np.array([r.bin for r in res]),
-            codePhaseRaw=np.array([r.codePhaseRaw for r in res]),
-            peak=np.array([r.peak for r in res]),
-            second=np.array([r.second for r in res]),
-        )
+        out = _results(res)
         if return_rows:
             out["rows"] = rows
         return out
@@ -128,6 +133,36 @@ class AcquisitionEngine:
         c = settings.to_c(part_index, part_count)
         check(self.L.gnssb200_acq_search(self.h, C.byref(c), d_iq_ptr, fmt, n_samples, d_rows_ptr, stream or None),
               "gnssb200_acq_search")
+
+    def search_batch_device(self, d_iq_ptr: int, stride: int, n_records: int, n_samples: int, settings: Settings, d_rows_ptr: int,
+                            fmt: int = abi.FMT_INT8_IQ, part_index: int = 0, part_count: int = 0, stream: int = 0):
+        """gnssb200_acq_search_batch: record r at d_iq_ptr + r*stride (stride 0: one record searched n_records times),
+        row tables [n_records][n_sv][n_bins] at d_rows_ptr.  Asynchronous on `stream`."""
+        c = settings.to_c(part_index, part_count)
+        check(self.L.gnssb200_acq_search_batch(self.h, C.byref(c), d_iq_ptr, stride, n_records, fmt, n_samples, d_rows_ptr,
+                                               stream or None), "gnssb200_acq_search_batch")
+
+    def acquisition_batch(self, d_iq_ptr: int, stride: int, n_records: int, n_samples: int, settings: Settings,
+                          fmt: int = abi.FMT_INT8_IQ, return_rows=False):
+        """acquisition() of n_records device-resident records in one batched search: one copy of all row tables to the
+        host, then the peak / second-peak / threshold logic per record.  Returns one dict per record."""
+        import torch
+
+        nb = self.num_bins(settings)
+        n_sv = len(settings.acqSatelliteList)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        d_rows = torch.empty(n_records * n_sv * nb * np.dtype(abi.ACQ_ROW_DTYPE).itemsize, dtype=torch.uint8, device=dev)
+        self.search_batch_device(d_iq_ptr, stride, n_records, n_samples, settings, d_rows.data_ptr(), fmt=fmt,
+                                 stream=torch.cuda.current_stream().cuda_stream)
+        rows = d_rows.cpu().numpy().view(abi.ACQ_ROW_DTYPE).reshape(n_records, n_sv, nb)
+        outs = []
+        for r in range(n_records):
+            res, _ = self.finalize(settings, rows[r])
+            out = _results(res)
+            if return_rows:
+                out["rows"] = rows[r]
+            outs.append(out)
+        return outs
 
     def finalize(self, settings: Settings, rows: np.ndarray):
         c = settings.to_c()
@@ -160,16 +195,7 @@ class AcquisitionEngine:
         dist.all_gather_into_tensor(gathered, rows, group=group)
         merged = merge_row_tables(gathered.cpu().numpy().view(abi.ACQ_ROW_DTYPE).reshape(world, n_sv * nb))
         res, _ = self.finalize(settings, merged)
-        out = dict(
-            carrFreq=np.array([r.carrFreq for r in res]),
-            codePhase=np.array([r.codePhase for r in res]),
-            peakMetric=np.array([r.peakMetric for r in res]),
-            freqChannel=np.array([r.sv for r in res]),
-            bin=np.array([r.bin for r in res]),
-            codePhaseRaw=np.array([r.codePhaseRaw for r in res]),
-            peak=np.array([r.peak for r in res]),
-            second=np.array([r.second for r in res]),
-        )
+        out = _results(res)
         if return_rows:
             out["rows"] = merged.reshape(n_sv, nb)
         return out

@@ -15,10 +15,13 @@
 //    ("base spectra") and every (sv, bin) row costs one multiply + one inverse FFT per block.
 //
 // Kernels (all use fft16k::ifft, 400 threads, one CTA per SM, transform resident in shared memory):
-//  acq_code_kernel  C[code][k]   = conj(fft(code))           = unnormalised inverse DFT of the real code
-//  acq_base_kernel  X[cls][b][k] = fft(sum_m s[n+mN] e^{i theta})  (wipe-off + fold + unpack fused in the loads)
-//  acq_rows_kernel  per (sv,bin): y = ifft(X[(k-shift) mod N] * C[k]); |y|^2/N^2; block choice or
+//  acq_code_kernel  C[code][k]      = conj(fft(code))           = unnormalised inverse DFT of the real code
+//  acq_base_kernel  X[r][cls][b][k] = fft(sum_m s_r[n+mN] e^{i theta})  (wipe-off + fold + unpack fused in the loads)
+//  acq_rows_kernel  per (record, sv, bin): y = ifft(X_r[(k-shift) mod N] * C[k]); |y|^2/N^2; block choice or
 //                   non-coherent sum in registers; max / first argmax / second peak outside +-1 chip.
+// A call searches R records with the same settings (gnssb200_acq_search_batch; the single-record entry point is R = 1):
+// the row descriptors, class increments and code spectra do not depend on the record, only the X base and the output
+// table do.
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -44,7 +47,7 @@ struct AcqWorkspace {
   int n_codes = 0, n_cls = 0, n_blocks = 0, n_rows = 0, n_bins = 0;
   int8_t *d_code_samples = nullptr;  // [n_codes][N]
   float2 *d_C = nullptr;             // [n_codes][N]
-  float2 *d_X = nullptr;             // [n_cls][n_blocks][N]
+  float2 *d_X = nullptr;             // [R][n_cls][n_blocks][N]
   size_t X_cap = 0;
   float2 *d_tw16k = nullptr, *d_tw800 = nullptr;
   AcqRowDesc *d_rows = nullptr;
@@ -84,12 +87,16 @@ acq_code_kernel(const int8_t *code_samples, float2 *C, Tables tb) {
       });
 }
 
-// grid = n_cls * n_blocks.  X = fft(x) = conj(ifft_unnorm(conj(x))),
+// grid = R * n_cls * n_blocks, record r at iq + r*rec_stride.  X = fft(x) = conj(ifft_unnorm(conj(x))),
 // x[n] = sum_{m<T} s[blk*T*N + n + m*N] * exp(+i*2*pi*f*(n+m*N)/fs)      (acquisition.sci:62-63,111,115-116)
 __global__ void __launch_bounds__(fft16k::THREADS, 1)
-acq_base_kernel(const uint8_t *iq, int fmt, int coh_ms, int n_blocks, const unsigned long long *cls_inc, float2 *X, Tables tb) {
+acq_base_kernel(const uint8_t *iq_base, size_t rec_stride, int fmt, int coh_ms, int n_cls, int n_blocks,
+                const unsigned long long *cls_inc, float2 *X, Tables tb) {
   extern __shared__ float2 sm[];
-  const int cls = blockIdx.x / n_blocks, blk = blockIdx.x % n_blocks;
+  const int per_rec = n_cls * n_blocks;
+  const int rec = blockIdx.x / per_rec, cb = blockIdx.x % per_rec;
+  const int cls = cb / n_blocks, blk = cb % n_blocks;
+  const uint8_t *iq = iq_base + (size_t)rec * rec_stride;
   const unsigned long long inc = cls_inc[cls];
   const long long base = (long long)blk * coh_ms * fft16k::N;
   float2 *out = X + (size_t)blockIdx.x * fft16k::N;
@@ -139,14 +146,17 @@ __device__ __forceinline__ unsigned long long block_max_key(unsigned long long k
 
 struct AcqRowsArgs {
   const AcqRowDesc *rows;
-  int n_rows;
-  const float2 *X;   // [cls][blocks][N]
+  int n_rows;        // descriptors per record; work item i = record i / n_rows, descriptor i % n_rows
+  int n_items;       // R * n_rows
+  size_t x_rec;      // elements of X per record: n_cls * n_blocks * N
+  size_t out_rec;    // rows of the output table per record: n_sv * n_bins
+  const float2 *X;   // [R][cls][blocks][N]
   const float2 *C;   // [code][N]
   int n_blocks;      // 2 (stock) or K (non-coherent)
   int noncoh;        // 0: keep the block with the larger maximum; 1: sum all blocks
   int chip;          // round(fs/codeFreqBasis): 16 GPS, 31 GLONASS
   int glonass_rule;  // middle-branch test '>=' (GLONASS) instead of '>' (GPS)
-  gnssb200_acq_row *out;
+  gnssb200_acq_row *out;  // [R][n_sv][n_bins]
   Tables tb;
 };
 
@@ -165,9 +175,11 @@ __global__ void __launch_bounds__(fft16k::THREADS, 1) acq_rows_kernel(const AcqR
   extern __shared__ float2 sm[];
   __shared__ unsigned long long red[16];
   const float scale = 1.0f / ((float)fft16k::N * (float)fft16k::N);  // Scilab ifft carries 1/N
-  for (int row = blockIdx.x; row < a.n_rows; row += gridDim.x) {
-    const AcqRowDesc d = a.rows[row];
+  for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
+    const int rec = item / a.n_rows;
+    const AcqRowDesc d = a.rows[item - rec * a.n_rows];
     const float2 *C = a.C + (size_t)d.code * fft16k::N;
+    const float2 *Xr = a.X + (size_t)rec * a.x_rec;
     float acc[fft16k::R3];
 #pragma unroll
     for (int kb = 0; kb < fft16k::R3; kb++) acc[kb] = 0.f;
@@ -175,7 +187,7 @@ __global__ void __launch_bounds__(fft16k::THREADS, 1) acq_rows_kernel(const AcqR
     int best_arg = 0, best_blk = 0;
     int my_tau0 = 0;
     for (int blk = 0; blk < a.n_blocks; blk++) {
-      const float2 *X = a.X + ((size_t)d.cls * a.n_blocks + blk) * fft16k::N;
+      const float2 *X = Xr + ((size_t)d.cls * a.n_blocks + blk) * fft16k::N;
       float mag[fft16k::R3];
       fft16k::ifft(
           sm, a.tb,
@@ -232,7 +244,7 @@ __global__ void __launch_bounds__(fft16k::THREADS, 1) acq_rows_kernel(const AcqR
       r.code_phase = best_arg;
       r.second = best_second;
       r.block = best_blk;
-      a.out[d.out_index] = r;
+      a.out[(size_t)rec * a.out_rec + d.out_index] = r;
     }
   }
 }
@@ -309,8 +321,24 @@ static bool same_code_setup(const gnssb200_acq_cfg &a, const gnssb200_acq_cfg &b
   return a.system == GNSSB200_SYS_GLONASS || memcmp(a.sv, b.sv, sizeof(int32_t) * a.n_sv) == 0;
 }
 
-extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *d_iq, int fmt, int64_t n_samples,
-                                   gnssb200_acq_row *d_rows_out, void *cuda_stream) {
+// cudaMalloc into a workspace slot; the slot is empty (nullptr, capacity 0) unless the allocation succeeded
+template <typename T>
+static cudaError_t ws_reserve(T *&p, size_t &cap, size_t n) {
+  if (n <= cap) return cudaSuccess;
+  cudaFree(p);
+  p = nullptr;
+  cap = 0;
+  const cudaError_t e = cudaMalloc(&p, n * sizeof(T));
+  if (e != cudaSuccess) {
+    p = nullptr;
+    return e;
+  }
+  cap = n;
+  return cudaSuccess;
+}
+
+extern "C" int gnssb200_acq_search_batch(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *d_iq, size_t record_stride_bytes,
+                                         int n_records, int fmt, int64_t n_samples, gnssb200_acq_row *d_rows_out, void *cuda_stream) {
   if (!h || !cfg || !d_iq || !d_rows_out) {
     gnssb200_set_error(-10, "gnssb200_acq_search: null argument", __FILE__, __LINE__);
     return -10;
@@ -327,6 +355,12 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
   if (cfg->n_sv <= 0 || cfg->n_sv > 64 || cfg->coh_ms <= 0 || n_samples < gnssb200_acq_samples_needed(cfg)) {
     gnssb200_set_error(-13, "gnssb200_acq_search: bad sv list / coherent time / record too short", __FILE__, __LINE__);
     return -13;
+  }
+  const size_t rec_bytes = fmt == GNSSB200_FMT_INT8_IQ ? (size_t)n_samples * 2 : ((size_t)n_samples + 1) / 2;
+  if (n_records < 1 || (record_stride_bytes != 0 && record_stride_bytes < rec_bytes)) {
+    gnssb200_set_error(-15, "gnssb200_acq_search_batch: n_records < 1, or a record stride shorter than n_samples in fmt",
+                       __FILE__, __LINE__);
+    return -15;
   }
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
@@ -350,10 +384,18 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
       const double ang = 2.0 * M_PI * b / fft16k::M;
       t2[b] = make_float2((float)cos(ang), (float)sin(ang));
     }
-    CUDA_TRY(cudaMalloc(&w.d_tw16k, t1.size() * sizeof(float2)));
-    CUDA_TRY(cudaMalloc(&w.d_tw800, t2.size() * sizeof(float2)));
-    CUDA_TRY(cudaMemcpy(w.d_tw16k, t1.data(), t1.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(w.d_tw800, t2.data(), t2.size() * sizeof(float2), cudaMemcpyHostToDevice));
+    size_t c1 = 0, c2 = 0;
+    cudaError_t e = ws_reserve(w.d_tw16k, c1, t1.size());
+    if (e == cudaSuccess) e = ws_reserve(w.d_tw800, c2, t2.size());
+    if (e == cudaSuccess) e = cudaMemcpyAsync(w.d_tw16k, t1.data(), t1.size() * sizeof(float2), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(w.d_tw800, t2.data(), t2.size() * sizeof(float2), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // pageable host vectors
+    if (e != cudaSuccess) {
+      cudaFree(w.d_tw16k);
+      cudaFree(w.d_tw800);
+      w.d_tw16k = w.d_tw800 = nullptr;
+      CUDA_TRY(e);
+    }
   }
   const Tables tb{w.d_tw16k, w.d_tw800};
   // ---- code spectra (cached per code setup) ----
@@ -375,10 +417,10 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
         samples[(size_t)c * N + i - 1] = chips[idx - 1];
       }
     }
-    cudaFree(w.d_code_samples);
-    cudaFree(w.d_C);
-    CUDA_TRY(cudaMalloc(&w.d_code_samples, samples.size()));
-    CUDA_TRY(cudaMalloc(&w.d_C, samples.size() * sizeof(float2)));
+    w.codes_valid = false;
+    size_t c1 = 0, c2 = 0;  // exact sizes: the spectra are rebuilt whenever the code setup changes
+    CUDA_TRY(ws_reserve(w.d_code_samples, c1, samples.size()));
+    CUDA_TRY(ws_reserve(w.d_C, c2, samples.size()));
     CUDA_TRY(cudaMemcpyAsync(w.d_code_samples, samples.data(), samples.size(), cudaMemcpyHostToDevice, st));
     acq_code_kernel<<<n_codes, fft16k::THREADS, smem, st>>>(w.d_code_samples, w.d_C, tb);
     CUDA_TRY(cudaGetLastError());
@@ -432,22 +474,12 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
     x -= floor(x);
     inc[c] = (unsigned long long)(x * 18446744073709551616.0);
   }
-  if ((size_t)n_cls > w.cls_cap) {
-    cudaFree(w.d_cls_inc);
-    CUDA_TRY(cudaMalloc(&w.d_cls_inc, sizeof(unsigned long long) * n_cls));
-    w.cls_cap = n_cls;
-  }
-  const size_t x_need = (size_t)n_cls * K * N;
-  if (x_need > w.X_cap) {
-    cudaFree(w.d_X);
-    CUDA_TRY(cudaMalloc(&w.d_X, x_need * sizeof(float2)));
-    w.X_cap = x_need;
-  }
-  if (rows.size() > w.rows_cap) {
-    cudaFree(w.d_rows);
-    CUDA_TRY(cudaMalloc(&w.d_rows, sizeof(AcqRowDesc) * rows.size()));
-    w.rows_cap = rows.size();
-  }
+  const int R = n_records;
+  const size_t x_rec = (size_t)n_cls * K * N;
+  // the workspace X holds the base spectra of every record of the call: R * n_cls * K * 128 KB
+  CUDA_TRY(ws_reserve(w.d_cls_inc, w.cls_cap, (size_t)n_cls));
+  CUDA_TRY(ws_reserve(w.d_X, w.X_cap, x_rec * R));
+  CUDA_TRY(ws_reserve(w.d_rows, w.rows_cap, rows.size()));
   CUDA_TRY(cudaMemcpyAsync(w.d_cls_inc, inc.data(), sizeof(unsigned long long) * n_cls, cudaMemcpyHostToDevice, st));
   if (!rows.empty())
     CUDA_TRY(cudaMemcpyAsync(w.d_rows, rows.data(), sizeof(AcqRowDesc) * rows.size(), cudaMemcpyHostToDevice, st));
@@ -458,15 +490,20 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
   w.n_bins = n_bins;
 
   CUDA_TRY(cudaEventRecord(h->ev0, st));
-  const int total_rows = cfg->n_sv * n_bins;
+  const size_t out_rec = (size_t)cfg->n_sv * n_bins;
+  const int total_rows = (int)(out_rec * R);
   acq_fill_rows_kernel<<<(total_rows + 255) / 256, 256, 0, st>>>(d_rows_out, total_rows);
-  acq_base_kernel<<<n_cls * K, fft16k::THREADS, smem, st>>>((const uint8_t *)d_iq, fmt, cfg->coh_ms, K, w.d_cls_inc, w.d_X, tb);
+  acq_base_kernel<<<R * n_cls * K, fft16k::THREADS, smem, st>>>((const uint8_t *)d_iq, record_stride_bytes, fmt, cfg->coh_ms, n_cls,
+                                                                 K, w.d_cls_inc, w.d_X, tb);
   CUDA_TRY(cudaGetLastError());
   h->launches += 2;
   if (!rows.empty()) {
     AcqRowsArgs a;
     a.rows = w.d_rows;
     a.n_rows = (int)rows.size();
+    a.n_items = a.n_rows * R;
+    a.x_rec = x_rec;
+    a.out_rec = out_rec;
     a.X = w.d_X;
     a.C = w.d_C;
     a.n_blocks = K;
@@ -477,13 +514,18 @@ extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *c
     a.tb = tb;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-    const int grid = std::min((int)rows.size(), sms);
+    const int grid = std::min(a.n_items, sms);
     acq_rows_kernel<<<grid, fft16k::THREADS, smem, st>>>(a);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
   }
   CUDA_TRY(cudaEventRecord(h->ev1, st));
   return 0;
+}
+
+extern "C" int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *d_iq, int fmt, int64_t n_samples,
+                                   gnssb200_acq_row *d_rows_out, void *cuda_stream) {
+  return gnssb200_acq_search_batch(h, cfg, d_iq, 0, 1, fmt, n_samples, d_rows_out, cuda_stream);
 }
 
 // acquisition.sci:145-191 on the complete (sv x bin) row table

@@ -5,6 +5,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <vector>
 
@@ -116,6 +117,63 @@ extern "C" void gnssb200_rx_cold_allocate(gnssb200_rx *rx, const gnssb200_cfg *c
       gnssb200_ch_code(rx, c, ch, c->glonass_code_ref);
     }
   }
+}
+
+// FFT acquisition results -> channels (definition in gnssb200.h; not in the reference)
+extern "C" int gnssb200_rx_acq_allocate(gnssb200_rx *rx, const gnssb200_cfg *c, const gnssb200_acq_cfg *acq,
+                                        const gnssb200_acq_result *res, int32_t ch_sv_out[GNSSB200_N_CHANNELS]) {
+  const char *bad = nullptr;
+  const bool glo = acq && acq->system == GNSSB200_SYS_GLONASS;
+  if (!rx || !c || !acq || !res || acq->n_sv < 1 || acq->n_sv > 64 || (acq->system != GNSSB200_SYS_GPS && !glo))
+    bad = "gnssb200_rx_acq_allocate: bad arguments";
+  else if (acq->samp_freq != c->samp_rate)
+    bad = "gnssb200_rx_acq_allocate: acquisition and receiver sampling rates differ";
+  else if (acq->IF != (glo ? c->glonass_carrier_if : c->gps_carrier_if))
+    bad = "gnssb200_rx_acq_allocate: acquisition and receiver IF differ";
+  else if (acq->code_freq != (glo ? c->glonass_code_f : c->gps_code_f))
+    bad = "gnssb200_rx_acq_allocate: acquisition and receiver code rates differ";
+  else if (glo && acq->IF_step != 562500.0)
+    bad = "gnssb200_rx_acq_allocate: GLONASS IF step must be 562.5 kHz";
+  for (int i = 0; !bad && !glo && i < acq->n_sv; i++)
+    if (acq->sv[i] < 1 || acq->sv[i] > 32) bad = "gnssb200_rx_acq_allocate: GPS PRN must be 1..32";
+  if (bad) {
+    gnssb200_set_error(-20, bad, __FILE__, __LINE__);
+    return -20;
+  }
+  std::vector<int> order;  // detected entries, strongest first, ties in list order
+  for (int i = 0; i < acq->n_sv; i++)
+    if (res[i].peakMetric > acq->threshold) order.push_back(i);
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return res[a].peakMetric > res[b].peakMetric; });
+  const int n = order.size() < NCH ? (int)order.size() : NCH;
+  int32_t prn[NCH];
+  for (int ch = 0; ch < NCH; ch++) {
+    prn[ch] = ch < n ? (glo ? GNSSB200_PRN_GLONASS : acq->sv[order[ch]]) : 0;
+    if (ch_sv_out) ch_sv_out[ch] = ch < n ? acq->sv[order[ch]] : 0;
+  }
+  gnssb200_rx_cold_allocate(rx, c, prn);
+  const double res_hz = c->clock_mult * c->samp_rate / pow(2.0, (double)c->carrier_nco_bits);
+  const int P = glo ? GLO_HALF_CHIPS : HALF_CHIPS;
+  for (int ch = 0; ch < n; ch++) {
+    const gnssb200_acq_result &r = res[order[ch]];
+    const int fch = glo ? acq->sv[order[ch]] : 0;
+    gnssb200_chan *k = &rx->chan[ch];
+    // carrier: the acquired frequency in NCO units
+    if (glo) k->carrier_cold_corr = (int64_t)fch * (int64_t)(562500.0 / res_hz);
+    const int64_t ref = (glo ? c->glonass_carrier_ref : c->gps_carrier_ref) + k->carrier_cold_corr;
+    k->carrier_freq = ref + llround((r.carrFreq - acq->IF - fch * acq->IF_step) / res_hz);
+    long long nf = llround((double)(k->carrier_freq - ref) / (double)c->d_freq);
+    nf = nf > k->search_max_f ? k->search_max_f : (nf < -k->search_max_f ? -k->search_max_f : nf);
+    k->n_freq = (int32_t)nf;
+    k->del_freq = nf > 0 ? (int32_t)(-2 * nf) : (int32_t)(1 - 2 * nf);
+    gnssb200_ch_carrier(rx, c, ch, k->carrier_freq);
+    // code: the prompt replica (one half chip ahead of early) meets chip 0 at delay a = cell + 1; start two cells before
+    const long long cell = llround((double)(r.codePhase - 1) * 2.0 * acq->code_freq / acq->samp_freq) % P;
+    const int a = (int)((cell + 1) % P);
+    const int k0 = a >= 2 ? a - 2 : 0;
+    gnssb200_ch_code_slew(rx, ch, k0);
+    k->codes = 0;  // a whole sweep of the bin at the acquired frequency before the search moves on
+  }
+  return n;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -99,6 +99,9 @@ def lib() -> C.CDLL:
         L.gnssb200_acq_search.argtypes = [vp, P(abi.AcqCfg), vp, C.c_int, i64, vp, vp]
         L.gnssb200_acq_finalize.argtypes = [P(abi.AcqCfg), vp, vp]
         L.gnssb200_acq_pcps_host.argtypes = [vp, P(abi.AcqCfg), vp, C.c_int, i64, vp, vp]
+    if hasattr(L, "gnssb200_acq_search_batch"):
+        L.gnssb200_acq_search_batch.argtypes = [vp, P(abi.AcqCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, vp, vp]
+        L.gnssb200_rx_acq_allocate.argtypes = [P(abi.Rx), P(abi.Cfg), P(abi.AcqCfg), vp, vp]
     _lib = L
     return L
 

@@ -137,6 +137,29 @@ class TrackingEngine:
         k.carrier_cold_corr = int(fch * int(562500.0 / res))
         self.ch_carrier(s, ch, self.cfg.glonass_carrier_ref + k.carrier_cold_corr)
 
+    def acq_allocate(self, s: int, result: dict, settings) -> list:
+        """gnssb200_rx_acq_allocate on the host copy of receiver `s` (freshly initialised): channels from one record's
+        acquisition result (a dict as AcquisitionEngine.acquisition returns it, for the same acquisition `settings`),
+        detected satellites strongest first.  Returns the PRN / frequency channel of each allocated channel."""
+        n_sv = len(settings.acqSatelliteList)
+        res = (abi.AcqResult * n_sv)()
+        for i in range(n_sv):
+            r = res[i]
+            r.carrFreq = float(result["carrFreq"][i])
+            r.codePhase = int(result["codePhase"][i])
+            r.sv = int(result["freqChannel"][i])
+            r.peakMetric = float(result["peakMetric"][i])
+            r.bin = int(result["bin"][i])
+            r.codePhaseRaw = int(result["codePhaseRaw"][i])
+            r.peak = float(result["peak"][i])
+            r.second = float(result["second"][i])
+        c = settings.to_c()
+        sv_out = (C.c_int32 * abi.N_CHANNELS)()
+        n = self.L.gnssb200_rx_acq_allocate(C.byref(self.rx[s]), C.byref(self.cfg), C.byref(c), res, sv_out)
+        if n < 0:
+            check(n, "gnssb200_rx_acq_allocate")
+        return [int(v) for v in sv_out[:n]]
+
     def upload(self):
         check(self.L.gnssb200_upload_rx(self.h, 0, self.n_streams, C.addressof(self.rx)), "gnssb200_upload_rx")
 

@@ -342,6 +342,18 @@ int64_t gnssb200_acq_samples_needed(const gnssb200_acq_cfg *cfg);
 int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *d_iq, int fmt,
                         int64_t n_samples, gnssb200_acq_row *d_rows, void *cuda_stream);
 
+/* The same search over R = n_records records with the same settings in one call (gnssb200_acq_search is the case
+ * R = 1).  Record r starts at d_iq + r*record_stride_bytes (0 = every record is the same buffer), e.g. the stream
+ * buffer that gnssb200_track_run then consumes; a non-zero stride must cover the bytes n_samples takes in fmt.
+ *   d_rows   device [R][n_sv][n_bins]: record r's table is laid out exactly like gnssb200_acq_search's, with the same
+ *            partition rule (part_index / part_count).
+ * The handle's workspace holds the base spectra of all R records: R * n_cls * K * 128 KB, n_cls = the number of
+ * distinct Doppler-bin frequencies modulo 1 kHz, K = 2 (stock) or n_noncoh -- 0.5 MB per record for 1 ms / 500 Hz
+ * bins, about 51 MB per record for 10 ms x 20 non-coherent / 50 Hz bins.  A failed allocation is returned as an error.
+ * Asynchronous on cuda_stream. */
+int gnssb200_acq_search_batch(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *d_iq, size_t record_stride_bytes,
+                              int n_records, int fmt, int64_t n_samples, gnssb200_acq_row *d_rows, void *cuda_stream);
+
 /* Peak / second-peak / threshold logic of acquisition.sci:145-191 on a complete host row table. */
 int gnssb200_acq_finalize(const gnssb200_acq_cfg *cfg, const gnssb200_acq_row *h_rows,
                           gnssb200_acq_result *results /* [n_sv] */);
@@ -349,6 +361,36 @@ int gnssb200_acq_finalize(const gnssb200_acq_cfg *cfg, const gnssb200_acq_row *h
 /* Convenience: host record in, results out (search + finalize, single GPU, synchronises). */
 int gnssb200_acq_pcps_host(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const void *h_iq, int fmt,
                            int64_t n_samples, gnssb200_acq_result *results, gnssb200_acq_row *h_rows_opt);
+
+/* Hand-off of one record's FFT acquisition results to the channels of the integer receiver.  The C reference has no
+ * such hand-off (its main starts channels with simple_cold_allocate and a PRN list fixed in advance, then searches
+ * serially); this is an extension of this library, defined as follows.
+ *
+ * rx must be freshly initialised (gnssb200_rx_init) for the record the acquisition ran on, starting at its sample 0.
+ * The detected entries (peakMetric > acq->threshold; FCH 0 counts) are ordered by peakMetric, strongest first, ties
+ * in list order, and at most 12 are kept -- the order of SCI/x/include/preRun.sci:66-81.  gnssb200_rx_cold_allocate
+ * gives entry i channel i (PRN register = the GPS PRN, or GNSSB200_PRN_GLONASS); the other channels stay off.  Then,
+ * with res = clock_mult*samp_rate/2^carrier_nco_bits, d = cfg->d_freq and llround() rounding halves away from 0:
+ *   carrier   GLONASS: carrier_cold_corr = fch * (int64)(562500/res), as for any GLONASS channel.
+ *             carrier_freq = ref + carrier_cold_corr + llround((carrFreq - IF - fch*IF_step) / res), ref the GPS or
+ *             GLONASS carrier reference word, written to the carrier NCO.  The channel confirms and pulls in from the
+ *             acquired frequency, whatever bin it is in (reference quirk Q2 does not arise).
+ *             n_freq = llround((carrier_freq - ref - carrier_cold_corr) / d) clamped to +-search_max_f,
+ *             del_freq = -2*n_freq (n_freq > 0) or 1 - 2*n_freq, as when the serial search enters bin n_freq.
+ *   code      tau = codePhase - 1 is the sample at which chip 0 starts.  Search cell k = llround(tau*2*code_f/fs) mod P
+ *             (P = 2046 half chips for GPS, 1022 for GLONASS; a satellite with code phase theta chips at sample 0 has
+ *             k = 2*(code_length - theta)).  The prompt replica runs one half chip ahead of early, so it meets chip 0
+ *             at code delay a = (k + 1) mod P.  The channel starts the serial search two cells before that:
+ *             k0 = a - 2 (0 when a < 2), written as code slew k0 -- the first period lasts P + k0 half chips, dump 1
+ *             tests delay k0, dump 2 delay k0 + 1, dump 3 delay a -- with codes = 0, so a whole sweep of the bin at
+ *             the acquired frequency follows if the satellite is missed.  Dump 0 always tests delay 0; a satellite
+ *             within a cell of it may be confirmed there first, fail the confirmation at delay k0 and be found
+ *             again a few dumps later.
+ * Returns the number of channels allocated (0..12), or < 0 -- rx untouched -- when acq and cfg disagree (sampling
+ * rate, IF, code rate, GLONASS IF step of 562.5 kHz) or an argument is invalid.  Channels 0..n-1 are allocated, the
+ * others stay off; ch_sv_out[12] (may be NULL) receives the PRN / FCH of each channel (0 for channels left off). */
+int gnssb200_rx_acq_allocate(gnssb200_rx *rx, const gnssb200_cfg *cfg, const gnssb200_acq_cfg *acq,
+                             const gnssb200_acq_result *res /* [acq->n_sv] */, int32_t ch_sv_out[GNSSB200_N_CHANNELS]);
 
 /* ---------------------------------------------------------------------------------------------
  * (2) batched layer -- floating-point tracking of the Scilab receivers (SURVEY.md 8f, rank 1)
