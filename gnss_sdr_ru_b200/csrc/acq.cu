@@ -18,7 +18,7 @@
 //  acq_code_kernel  C[code][k]      = conj(fft(code))           = unnormalised inverse DFT of the real code
 //  acq_base_kernel  X[r][cls][b][k] = fft(sum_m s_r[n+mN] e^{i theta})  (wipe-off + fold + unpack fused in the loads)
 //  acq_rows_kernel  per (record, sv, bin): y = ifft(X_r[(k-shift) mod N] * C[k]); |y|^2/N^2; block choice or
-//                   non-coherent sum in registers; max / first argmax / second peak outside +-1 chip.
+//                   non-coherent sum in registers; max / first argmax / second peak at circular distance >= 1 chip.
 // A call searches R records with the same settings (gnssb200_acq_search_batch; the single-record entry point is R = 1):
 // the row descriptors, class increments and code spectra do not depend on the record, only the X base and the output
 // table do.
@@ -155,20 +155,17 @@ struct AcqRowsArgs {
   int n_blocks;      // 2 (stock) or K (non-coherent)
   int noncoh;        // 0: keep the block with the larger maximum; 1: sum all blocks
   int chip;          // round(fs/codeFreqBasis): 16 GPS, 31 GLONASS
-  int glonass_rule;  // middle-branch test '>=' (GLONASS) instead of '>' (GPS)
   gnssb200_acq_row *out;  // [R][n_sv][n_bins]
   Tables tb;
 };
 
-// is 0-based code phase t searched for the second peak, given the peak at 0-based p?
-// (acquisition.sci:151-168; 1-based there)
-__device__ __forceinline__ bool second_peak_allowed(int t, int p, int chip, int glonass_rule) {
-  const int n = fft16k::N;
-  const int e1 = p + 1 - chip, e2 = p + 1 + chip;  // 1-based excludeRangeIndex1/2
-  const int t1 = t + 1;
-  if (e1 < 2) return t1 >= e2 && t1 <= n + e1;
-  if (glonass_rule ? (e2 >= n) : (e2 > n)) return t1 >= e2 - n && t1 <= e1;
-  return t1 <= e1 || t1 >= e2;
+// is 0-based code phase t searched for the second peak, given the peak at 0-based p?  Circular distance >= chip:
+// the window of acquisition.sci:151-168 at every peak where its index ranges stay inside 1..N.  At the three peaks
+// where they do not (1-based GPS 17, GLONASS 32 and 15969; Scilab stops with an error) this is an extension of the
+// library: the same circular rule.
+__device__ __forceinline__ bool second_peak_allowed(int t, int p, int chip) {
+  const int d = abs(t - p);
+  return min(d, fft16k::N - d) >= chip;
 }
 
 __global__ void __launch_bounds__(fft16k::THREADS, 1) acq_rows_kernel(const AcqRowsArgs a) {
@@ -218,12 +215,12 @@ __global__ void __launch_bounds__(fft16k::THREADS, 1) acq_rows_kernel(const AcqR
       key = block_max_key(key, red);
       const float peak = __uint_as_float((unsigned)(key >> 32));
       const int arg = 0x7fffffff - (int)(unsigned)(key & 0xffffffffu);
-      // second peak outside +-1 chip around this row's own peak
+      // second peak at circular distance >= 1 chip from this row's own peak
       unsigned long long key2 = 0;
 #pragma unroll
       for (int kb = 0; kb < fft16k::R3; kb++) {
         const int t = my_tau0 + 400 * kb;
-        if (second_peak_allowed(t, arg, a.chip, a.glonass_rule)) {
+        if (second_peak_allowed(t, arg, a.chip)) {
           const unsigned long long k2 = pack_key(mag[kb], t);
           key2 = k2 > key2 ? k2 : key2;
         }
@@ -509,7 +506,6 @@ extern "C" int gnssb200_acq_search_batch(gnssb200_handle *h, const gnssb200_acq_
     a.n_blocks = K;
     a.noncoh = cfg->n_noncoh >= 2 ? 1 : 0;
     a.chip = scilab_round(cfg->samp_freq / cfg->code_freq);
-    a.glonass_rule = cfg->system == GNSSB200_SYS_GLONASS ? 1 : 0;
     a.out = d_rows_out;
     a.tb = tb;
     int sms = 148;

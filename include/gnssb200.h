@@ -295,7 +295,7 @@ int gnssb200_synth(gnssb200_handle *h, void *d_out, size_t stream_stride_bytes, 
 #define GNSSB200_SYS_GLONASS 1
 
 typedef struct gnssb200_acq_cfg {
-  int32_t system;           /* GNSSB200_SYS_* : code table + exclusion-window rule (GPS '>' / GLONASS '>=') */
+  int32_t system;           /* GNSSB200_SYS_* : code table and chip length of the second-peak window */
   double samp_freq;         /* settings.samplingFreq   16e6 */
   double IF;                /* settings.IF             GPS 2.42e6 / GLONASS 1e6 */
   double IF_step;           /* settings.L1_IF_step     GLONASS 562500, GPS 0 */
@@ -315,7 +315,10 @@ typedef struct gnssb200_acq_cfg {
 typedef struct gnssb200_acq_row {   /* one (sv, Doppler bin) row of the search grid */
   float peak;               /* max over code phases of the kept block */
   int32_t code_phase;       /* 0-based first argmax (Scilab's is this + 1) */
-  float second;             /* max outside +-1 chip around this row's own argmax (reference rule) */
+  float second;             /* max over the code phases at circular distance >= 1 chip (16 GPS / 31 GLONASS samples)
+                             * from this row's own argmax: the window of acquisition.sci:151-168 wherever its index
+                             * ranges stay inside 1..N.  At 1-based argmax 17 (GPS), 32 and 15969 (GLONASS) they
+                             * do not and Scilab stops; there the same circular rule is an extension of this library */
   int32_t block;            /* which block was kept (0/1); 0 for non-coherent mode */
 } gnssb200_acq_row;
 

@@ -18,6 +18,15 @@ wipe-off + FFT per bin), not the folded / spectrum-shift formulation of the CUDA
 Non-coherent mode (n_noncoh >= 2, BASELINE config 4) is NOT in the Scilab code (which keeps the
 better of two blocks); it is defined here as the sum over K consecutive Tcoh-ms blocks of
 abs(ifft(...))^2 with the same per-block wipe-off, no data-bit handling.
+
+Second-peak window (extension).  acquisition.sci:151-168 searches the second peak over the code phases at circular
+distance >= chip = round(fs/codeFreqBasis) from the peak P (1-based), written as three index ranges.  At 31997 of the
+32000 (system, P) positions that is exactly second_peak_window(); at GPS P = 17 and GLONASS P = 32 and 15969 the
+reference's range leaves 1..N and Scilab stops with an error (exclusion_range restates the ranges as written).  This
+library defines those three positions by the circular rule the reference follows everywhere else:
+acquisition(..., undefined="circular").  The default, undefined="raise", raises as the reference does.  The per-row
+seconds of acquisition()'s "row_second" (the reference computes the second peak of the winning row only) use the
+circular rule at every position, as the CUDA path does for every row.
 """
 from __future__ import annotations
 
@@ -96,6 +105,12 @@ def samples_needed(s: AcqSettings) -> int:
 
 def acquisition_rows(longSignal: np.ndarray, s: AcqSettings, sv: int, bins=None):
     """results(frqBinIndex,:) for one sv, reduced to per-row (max, first argmax 0-based, block)."""
+    rows, full, _ = _rows(longSignal, s, sv, bins)
+    return rows, full
+
+
+def _rows(longSignal, s, sv, bins=None):
+    """acquisition_rows plus, per row, the maximum of every block (stock mode: the two the '>' compares)."""
     n = samples_per_code(s)
     T = s.acqCohIntegration
     L = T * n
@@ -109,6 +124,7 @@ def acquisition_rows(longSignal: np.ndarray, s: AcqSettings, sv: int, bins=None)
     blocks = [longSignal[k * L:(k + 1) * L] for k in range(K)]
     rows = {}
     full = {}
+    block_max = {}
     for k1 in bins:
         f = bin_freq(s, sv, k1)
         sigCarr = np.exp(1j * f * phasePoints)
@@ -124,7 +140,8 @@ def acquisition_rows(longSignal: np.ndarray, s: AcqSettings, sv: int, bins=None)
             row = np.sum(res, axis=0)[:n]
         rows[k1] = (float(row.max()), int(np.argmax(row)), blk_idx)
         full[k1] = row
-    return rows, full
+        block_max[k1] = tuple(float(r[:n].max()) for r in res)
+    return rows, full, block_max
 
 
 def exclusion_range(s: AcqSettings, codePhase1: int) -> np.ndarray:
@@ -143,6 +160,21 @@ def exclusion_range(s: AcqSettings, codePhase1: int) -> np.ndarray:
     return rng
 
 
+def second_peak_window(s: AcqSettings, codePhase1: int) -> np.ndarray:
+    """1-based code-phase indices at circular distance >= chip from the 1-based peak codePhase1: the window of
+    exclusion_range wherever that range lies inside 1..N, and this library's definition where it does not."""
+    n = samples_per_code(s)
+    chip = int(np.floor(s.samplingFreq / s.codeFreqBasis + 0.5))
+    d = np.abs(np.arange(1, n + 1) - codePhase1)
+    return np.flatnonzero(np.minimum(d, n - d) >= chip) + 1
+
+
+def row_seconds(s: AcqSettings, rows: dict, full: dict) -> dict:
+    """Per row: the largest value inside second_peak_window around that row's own argmax (what the CUDA path stores
+    as a row's `second`)."""
+    return {k1: float(full[k1][second_peak_window(s, rows[k1][1] + 1) - 1].max()) for k1 in rows}
+
+
 def acquisition_job(job):
     """(int8 I,Q record, settings) -> acquisition(): a picklable entry point so that tests can run one code entry per
     process (BASELINE config 4 needs about two minutes per PRN in this formulation)."""
@@ -150,12 +182,18 @@ def acquisition_job(job):
     return acquisition(to_complex(rec), s)
 
 
-def acquisition(longSignal: np.ndarray, s: AcqSettings):
+def acquisition(longSignal: np.ndarray, s: AcqSettings, undefined: str = "raise"):
     """acqResults = acquisition(longSignal, settings).  Returns a list of dicts (one per sv) with
-    the reference's fields plus the raw peak data."""
+    the reference's fields plus the raw peak data: "rows" {bin: (peak, argmax, block)}, "row_second" {bin: second
+    peak of that row} and "row_block_max" {bin: maximum of each block}.
+    undefined: what a peak at one of the three positions whose exclusion range leaves 1..N gives -- "raise" (the
+    reference stops there) or "circular" (second_peak_window, this library's definition)."""
+    if undefined not in ("raise", "circular"):
+        raise ValueError(undefined)
+    n = samples_per_code(s)
     out = []
     for sv in s.svList:
-        rows, full = acquisition_rows(longSignal, s, sv)
+        rows, full, block_max = _rows(longSignal, s, sv)
         nb = num_bins(s)
         rowmax = np.array([rows[k][0] for k in range(1, nb + 1)])
         peak = rowmax.max()
@@ -163,12 +201,15 @@ def acquisition(longSignal: np.ndarray, s: AcqSettings):
         colmax = np.max(np.stack([full[k] for k in range(1, nb + 1)]), axis=0)
         codePhase = int(np.argmax(colmax)) + 1  # first column attaining it (:148)
         rng = exclusion_range(s, codePhase)
-        if rng.min() < 1:
-            raise IndexError("Scilab would raise: exclusion range touches index 0 (acquisition.sci:163)")
+        if rng.min() < 1 or rng.max() > n:
+            if undefined == "raise":
+                raise IndexError(f"Scilab would raise: exclusion range of peak {codePhase} leaves 1..{n} (acquisition.sci:151-168)")
+            rng = second_peak_window(s, codePhase)
         second = float(full[frequencyBinIndex][rng - 1].max())
         metric = peak / second
         r = dict(sv=sv, peakMetric=metric, bin=frequencyBinIndex, codePhaseRaw=codePhase, peak=float(peak),
-                 second=second, carrFreq=0.0, codePhase=0, freqChannel=0, rows=rows)
+                 second=second, carrFreq=0.0, codePhase=0, freqChannel=0, rows=rows,
+                 row_second=row_seconds(s, rows, full), row_block_max=block_max)
         if metric > s.acqThreshold:
             r["codePhase"] = codePhase
             r["carrFreq"] = bin_freq(s, sv, frequencyBinIndex)

@@ -118,8 +118,9 @@ def test_more_than_twelve_detections(oracle_lib):
 
 
 def test_none_detected(oracle_lib):
-    st = _gps([1, 2, 3])
-    n, rx, sv = _check(oracle_lib, st, [(0.0, 0, 1.5), (0.0, 0, 2.9), (0.0, 0, 3.0)])  # 3.0 is not > 3.0
+    st = _gps([1, 2, 3, 4])
+    # 3.0 is not > 3.0; NaN (0/0 of an all-zero record) is not either
+    n, rx, sv = _check(oracle_lib, st, [(0.0, 0, 1.5), (0.0, 0, 2.9), (0.0, 0, 3.0), (0.0, 0, math.nan)])
     assert n == 0 and sv == [0] * 12
     assert all(rx.reg_write[ch << 3] == 0 for ch in range(12))  # every channel off
 

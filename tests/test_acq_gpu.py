@@ -19,6 +19,7 @@ def _check(res, ora, rows_gpu, nb, check_rows=True):
         assert int(res["codePhaseRaw"][i]) == o["codePhaseRaw"], (i, res["codePhaseRaw"][i], o["codePhaseRaw"])
         assert abs(res["peakMetric"][i] - o["peakMetric"]) <= RTOL * o["peakMetric"], (i, res["peakMetric"][i], o["peakMetric"])
         assert abs(res["peak"][i] - o["peak"]) <= RTOL * o["peak"]
+        assert abs(res["second"][i] - o["second"]) <= RTOL * o["second"]
         assert int(res["codePhase"][i]) == o["codePhase"]
         assert int(res["freqChannel"][i]) == o["freqChannel"]
         assert res["carrFreq"][i] == o["carrFreq"]
@@ -29,6 +30,12 @@ def _check(res, ora, rows_gpu, nb, check_rows=True):
                 assert abs(g["peak"] - pk) <= RTOL * pk, (i, b, g["peak"], pk)
                 # argmax / block must agree unless two maxima tie within fp32 noise
                 assert int(g["code_phase"]) == arg or abs(g["peak"] - pk) <= 1e-6 * pk, (i, b, g, arg)
+                bm = o["row_block_max"][b + 1]
+                assert int(g["block"]) == blk or (len(bm) == 2 and abs(bm[0] - bm[1]) <= 1e-5 * max(bm)), (i, b, g, blk, bm)
+                # the second peak of the row, in the window around the row's own argmax
+                if int(g["code_phase"]) == arg and int(g["block"]) == blk:
+                    s2 = o["row_second"][b + 1]
+                    assert abs(g["second"] - s2) <= RTOL * s2, (i, b, g["second"], s2)
 
 
 def test_gps_acq_1ms(oracle_lib):

@@ -43,6 +43,49 @@ def test_exclusion_ranges(oracle_lib):
     assert po.exclusion_range(g, 5000)[-1] == n and 5031 in po.exclusion_range(g, 5000) and 5030 not in po.exclusion_range(g, 5000)
 
 
+def test_second_peak_window_is_the_reference_range_except_at_three_positions(oracle_lib):
+    """For every peak position P of both systems, the circular window (distance >= chip) equals the reference's
+    exclusion range, except at the three positions where that range leaves 1..N (Scilab stops there; this library
+    defines them by the circular rule).  A change of either rule shows up in the list below."""
+    from oracle import pcps_oracle as po
+
+    n = 16000
+    undefined = []
+    for s in (po.AcqSettings.gps(), po.AcqSettings.glonass()):
+        chip = 16 if s.system == "gps" else 31
+        for P in range(1, n + 1):
+            w = po.second_peak_window(s, P)
+            r = po.exclusion_range(s, P)
+            if r.min() < 1 or r.max() > n:
+                undefined.append((s.system, P))
+                assert len(r) == len(w) and not np.array_equal(r, w)  # the same count, one index outside 1..N
+            else:
+                assert np.array_equal(np.sort(r), w), (s.system, P)
+            assert len(w) == n - 2 * chip + 1
+    assert undefined == [("gps", 17), ("glonass", 32), ("glonass", 15969)]
+
+
+def test_undefined_positions_raise_or_follow_the_circular_rule(oracle_lib):
+    """A peak at GPS P = 17 raises by default, as the reference does; undefined="circular" gives the second peak
+    over second_peak_window, which holds sample 1 (circular distance 16 from the peak)."""
+    import pytest
+
+    from oracle import pcps_oracle as po
+
+    s = po.AcqSettings.gps(acqSearchBand=1.0, acqCohIntegration=1, svList=[1])
+    c = po.sampled_code(s, 1)
+    n = np.arange(2 * 16000)
+    # peak at 1-based 17, echo at 1, on the carrier of the middle bin (the wipe-off multiplies by exp(+i*2*pi*f*t))
+    x = np.tile(np.roll(c, 16) * 40 + c * 20, 2) * np.exp(-2j * np.pi * s.IF * n / s.samplingFreq)
+    with pytest.raises(IndexError):
+        po.acquisition(x, s)
+    r = po.acquisition(x, s, undefined="circular")[0]
+    assert r["codePhaseRaw"] == 17
+    full = po.acquisition_rows(x, s, 1)[1][r["bin"]]
+    assert r["second"] == full[0] and r["second"] == max(full[po.second_peak_window(s, 17) - 1])
+    assert r["row_second"][r["bin"]] == r["second"]
+
+
 def test_oracle_regression_fixture(oracle_lib):
     from oracle import pcps_oracle as po
 
