@@ -47,6 +47,7 @@ struct gnssb200_handle {
   int32_t *d_chan_flags;      // [n_streams*12] bit0: dumped in the last block, bit1: halted
   long long track_slice;      // blocks per work-queue slice of the tracking kernel; 0 = automatic (gnssb200_set_track_slice)
   int track_form, track_occ;  // kernel form / occupancy variant forced by gnssb200_set_track_variant (0 = automatic)
+  int softtrack_width;        // threads per channel of gnssb200_softtrack_batch (gnssb200_set_softtrack_width; 0 = automatic)
   void *d_sched;              // work queue of track_ws_kernel: headers / TIC counters / slots / dump counters per channel
   uint32_t *d_code_table;     // [TABLE_ENTRIES+1] packed E | P<<8 | L<<16 (int8 each), last entry 0
   int8_t *d_chips;            // [33][1024] chips as +-1: row 0 GLONASS ST code, rows 1..32 GPS C/A (chip_table, synth.cu)

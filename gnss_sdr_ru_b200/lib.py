@@ -102,6 +102,10 @@ def lib() -> C.CDLL:
     if hasattr(L, "gnssb200_acq_search_batch"):
         L.gnssb200_acq_search_batch.argtypes = [vp, P(abi.AcqCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, vp, vp]
         L.gnssb200_rx_acq_allocate.argtypes = [P(abi.Rx), P(abi.Cfg), P(abi.AcqCfg), vp, vp]
+    if hasattr(L, "gnssb200_softtrack_batch"):
+        L.gnssb200_softtrack_batch.argtypes = [vp, P(abi.SoftTrackCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, vp, vp, C.c_int,
+                                               vp, vp, vp]
+        L.gnssb200_set_softtrack_width.argtypes = [vp, C.c_int]
     _lib = L
     return L
 

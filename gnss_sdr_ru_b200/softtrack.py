@@ -65,6 +65,16 @@ def preRun(acqResults: dict, settings: TrackSettings) -> list:
                  codePhase=int(acqResults["codePhase"][i]), status="T") for i in order[:n]]
 
 
+def _track_results(out: np.ndarray, done: np.ndarray, channel: list) -> list:
+    """trackResults dicts of the rows [n_ch][ms][13] and periods done [n_ch] of the channels in `channel`."""
+    res = []
+    for i, c in enumerate(channel):
+        r = {f: out[i, : done[i], k].copy() for k, f in enumerate(abi.SOFTTRACK_FIELDS)}
+        r["SVN"], r["FCH"], r["status"] = c.get("SVN", 0), c["FCH"], c.get("status", "T")
+        res.append(r)
+    return res
+
+
 class SoftTrackingEngine:
     def __init__(self, device: int = 0, handle=None):
         self.L = lib()
@@ -109,14 +119,53 @@ class SoftTrackingEngine:
         d_out = torch.zeros((n_ch, settings.msToProcess, 13), dtype=torch.float64, device="cuda")
         d_done = torch.zeros(n_ch, dtype=torch.int32, device="cuda")
         self.tracking_device(d_iq.data_ptr(), buf.size // 2, channel, settings, d_out.data_ptr(), d_done.data_ptr())
-        out = d_out.cpu().numpy()
-        done = d_done.cpu().numpy()
-        res = []
-        for i, c in enumerate(channel):
-            r = {f: out[i, : done[i], k].copy() for k, f in enumerate(abi.SOFTTRACK_FIELDS)}
-            r["SVN"], r["FCH"], r["status"] = c.get("SVN", 0), c["FCH"], c.get("status", "T")
-            res.append(r)
+        return _track_results(d_out.cpu().numpy(), d_done.cpu().numpy(), channel)
+
+    def tracking_batch_device(self, d_iq_ptr: int, stride: int, n_records: int, n_samples: int, channels: list,
+                              settings: TrackSettings, d_out_ptr: int, d_ms_done_ptr: int, fmt: int = abi.FMT_INT8_IQ,
+                              stream: int = 0):
+        """gnssb200_softtrack_batch: record r at d_iq_ptr + r*stride (stride 0: one record n_records times) in fmt
+        (FMT_INT8_IQ or FMT_PACKED2).  channels holds one preRun channel list per record; they are tracked as one
+        flat list, record by record, into d_out [n_ch][msToProcess][13] and d_ms_done [n_ch].  Synchronous on `stream`."""
+        if len(channels) != n_records:
+            raise ValueError("channels must hold one channel list per record")
+        flat = [(r, c) for r, chl in enumerate(channels) for c in chl]
+        ch = (abi.SoftTrackChan * len(flat))()
+        rec = (C.c_int32 * len(flat))()
+        for i, (r, c) in enumerate(flat):
+            ch[i].sv = c["FCH"]
+            ch[i].code_phase = c["codePhase"]
+            ch[i].acquired_freq = c["acquiredFreq"]
+            rec[i] = r
+        cfg = settings.to_c()
+        check(self.L.gnssb200_softtrack_batch(self.h, C.byref(cfg), d_iq_ptr, stride, n_records, fmt, n_samples, ch, rec, len(flat),
+                                              d_out_ptr, d_ms_done_ptr, stream or None), "gnssb200_softtrack_batch")
+
+    def tracking_batch(self, d_iq_ptr: int, stride: int, n_records: int, n_samples: int, channels: list, settings: TrackSettings,
+                       fmt: int = abi.FMT_INT8_IQ) -> list:
+        """tracking() of n_records device-resident records in one call: one list of trackResults dicts per record."""
+        import torch
+
+        n_ch = sum(len(chl) for chl in channels)
+        if len(channels) != n_records:
+            raise ValueError("channels must hold one channel list per record")
+        if n_ch == 0:
+            return [[] for _ in channels]
+        dev = torch.device("cuda", torch.cuda.current_device())
+        d_out = torch.zeros((n_ch, settings.msToProcess, 13), dtype=torch.float64, device=dev)
+        d_done = torch.zeros(n_ch, dtype=torch.int32, device=dev)
+        self.tracking_batch_device(d_iq_ptr, stride, n_records, n_samples, channels, settings, d_out.data_ptr(), d_done.data_ptr(),
+                                   fmt=fmt, stream=torch.cuda.current_stream().cuda_stream)
+        out, done = d_out.cpu().numpy(), d_done.cpu().numpy()
+        res, i = [], 0
+        for chl in channels:
+            res.append(_track_results(out[i : i + len(chl)], done[i : i + len(chl)], chl))
+            i += len(chl)
         return res
+
+    def set_width(self, threads: int):
+        """Threads per channel of the batched call: 0 automatic, 128, 256 or 512.  Results do not depend on it."""
+        check(self.L.gnssb200_set_softtrack_width(self.h, threads), "gnssb200_set_softtrack_width")
 
     def last_kernel_ms(self) -> float:
         return float(self.L.gnssb200_last_kernel_ms(self.h))

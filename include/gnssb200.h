@@ -431,6 +431,25 @@ int gnssb200_softtrack(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, co
                        const gnssb200_softtrack_chan *chans, int n_ch, double *d_out, int32_t *d_ms_done,
                        void *cuda_stream);
 
+/* The float tracking of gnssb200_softtrack for channels spread over R = n_records records with the same settings.
+ * Record r starts at d_iq + r*record_stride_bytes (0: every record is the same buffer) and holds n_samples complex
+ * samples in fmt (INT8_IQ or PACKED2); a non-zero stride must cover them.  Channel i reads record chan_record[i]:
+ * it starts at cfg->skip_samples + chans[i].code_phase - 1 of that record and stops at that record's end.
+ * d_out [n_ch][ms_to_process][13] and d_ms_done [n_ch] are laid out exactly as gnssb200_softtrack's, and each
+ * channel's values are bit-identical to gnssb200_softtrack on its record alone (after unpacking, for PACKED2),
+ * whatever kernel width runs.  Returns < 0 and writes nothing to d_out / d_ms_done when an argument is invalid
+ * (n_records < 1, a chan_record out of range, another fmt, a stride that does not cover a record, a GPS PRN outside
+ * 1..32, a code length other than 511 / 1023, n_ch <= 0).  Synchronous on cuda_stream. */
+int gnssb200_softtrack_batch(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq,
+                             size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
+                             const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
+                             double *d_out, int32_t *d_ms_done, void *cuda_stream);
+
+/* Threads per channel of gnssb200_softtrack_batch: 0 automatic, else 128, 256 or 512.  Results do not depend on it.
+ * Automatic: the width whose CTAs finish all channels in the fewest waves, weighted by the measured time of a wave at
+ * that width -- 512 while every channel has an SM of its own, narrower beyond that (DESIGN §4.3). */
+int gnssb200_set_softtrack_width(gnssb200_handle *h, int threads);
+
 /* ---------------------------------------------------------------------------------------------
  * (2) batched layer -- streaming ingest (SURVEY.md 8f, rank 4): a circular buffer between a sample
  *     producer and the GPU channel loop of ONE stream of the handle, modelled on
