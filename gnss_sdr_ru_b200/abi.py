@@ -217,6 +217,19 @@ class SoftTrackChan(C.Structure):
     _fields_ = [("sv", C.c_int32), ("code_phase", C.c_int32), ("acquired_freq", C.c_double)]
 
 
+class SoftTrackState(C.Structure):
+    """gnssb200_softtrack_state: one float-tracking channel between two code periods."""
+    _fields_ = [("codeFreq", C.c_double), ("remCodePhase", C.c_double), ("carrFreq", C.c_double), ("remCarrPhase", C.c_double),
+                ("oldCodeNco", C.c_double), ("oldCodeError", C.c_double), ("oldCarrNco", C.c_double), ("oldCarrError", C.c_double),
+                ("I1", C.c_double), ("Q1", C.c_double), ("carrFreqBasis", C.c_double), ("pos", C.c_int64), ("sv", C.c_int32),
+                ("record", C.c_int32), ("ms_done", C.c_int32), ("status", C.c_int32)]
+
+
+# gnssb200_softtrack_state.status
+SOFTTRACK_RUNNING, SOFTTRACK_RECORD_END, SOFTTRACK_MS_DONE = 0, 1, 2
+SOFTTRACK_BEHIND, SOFTTRACK_BAD_RECORD, SOFTTRACK_BAD_SV = -1, -2, -3
+
+
 class IngestStat(C.Structure):
     _fields_ = [("bytes_loaded", C.c_int64), ("bytes_output", C.c_int64), ("bytes_in_buffer", C.c_int64), ("ring_bytes", C.c_int64),
                 ("blocks_done", C.c_int64), ("finished", C.c_int32), ("overflow", C.c_int32)]

@@ -24,21 +24,15 @@
 #define FTRK_LANES 512
 #define FTRK_WARPS (FTRK_LANES / 32)
 
-struct FtrkChanDev {
-  int sv;               // PRN (GPS) or frequency channel (GLONASS)
-  int code_row;         // row in the chip table (0: GLONASS ST code, 1..32: C/A)
-  double acquired_freq;
-  long long start;      // first complex sample of the channel in its record (skip + codePhase - 1)
-  long long rec_off;    // byte offset of the channel's record from FtrkArgs::iq
-};
-
 struct FtrkArgs {
-  const uint8_t *iq;
-  long long n_samples;  // of every record
+  const uint8_t *win;   // record r's window at win + r*win_stride; sample k at offset k - win_first (DESIGN §4.3)
+  size_t win_stride;
+  int n_records;
+  long long win_first, win_end, record_samples;
   const int8_t *chips;  // [33][1024]
-  const FtrkChanDev *chan;
+  gnssb200_softtrack_state *state;  // [n_ch]
   double *out;          // [n_ch][ms][13]
-  int32_t *ms_done;     // [n_ch]
+  int32_t *ms_done;     // [n_ch] or NULL: the one-shot calls' copy of state.ms_done
   int ms;
   int glonass;
   int code_len;
@@ -49,8 +43,10 @@ struct FtrkArgs {
 struct FtrkState {
   double codeFreq, remCodePhase, carrFreq, remCarrPhase;
   long long pos;
+  const uint8_t *rec;
   int blksize;
-  int stop;
+  int run;
+  int code_row;
 };
 
 __device__ __forceinline__ double warp_sum_d(double v) {
@@ -58,8 +54,9 @@ __device__ __forceinline__ double warp_sum_d(double v) {
   return v;
 }
 
-// complex sample k of a record: int8 I,Q, or the packed nibble (byte[k>>1] >> 4*(k&1)) & 15 with I in bits 0-1 and
-// Q in bits 2-3, code {0:+1, 1:-1, 2:+3, 3:-3} (DESIGN §3, sample_at in acq.cu)
+// complex sample k of a window (k counted from the window's first sample, which is even for packed input): int8 I,Q,
+// or the packed nibble (byte[k>>1] >> 4*(k&1)) & 15 with I in bits 0-1 and Q in bits 2-3, code {0:+1, 1:-1, 2:+3,
+// 3:-3} (DESIGN §3, sample_at in acq.cu)
 template <int FMT>
 __device__ __forceinline__ void ftrk_sample(const uint8_t *rec, long long k, double &I, double &Q) {
   if (FMT == GNSSB200_FMT_PACKED2) {
@@ -73,6 +70,17 @@ __device__ __forceinline__ void ftrk_sample(const uint8_t *rec, long long k, dou
   }
 }
 
+// What a channel does next, from its state between two periods: GNSSB200_SOFTTRACK_* and whether it runs the block
+// [pos, pos + blksize) now (only RUNNING channels whose block lies inside the window do).
+__device__ __forceinline__ int ftrk_next(const FtrkArgs &a, long long pos, int blksize, int ms_done, int *run) {
+  *run = 0;
+  if (ms_done >= a.ms) return GNSSB200_SOFTTRACK_MS_DONE;
+  if (pos < a.win_first) return GNSSB200_SOFTTRACK_BEHIND;
+  if (pos + blksize > a.record_samples) return GNSSB200_SOFTTRACK_RECORD_END;
+  *run = pos + blksize <= a.win_end;
+  return GNSSB200_SOFTTRACK_RUNNING;
+}
+
 template <int NT, int FMT>
 __global__ void __launch_bounds__(NT) softtrack_kernel(const FtrkArgs a) {
   static_assert(FTRK_LANES % NT == 0 && NT % 32 == 0, "a CTA runs whole warps of virtual lanes");
@@ -80,36 +88,59 @@ __global__ void __launch_bounds__(NT) softtrack_kernel(const FtrkArgs a) {
   __shared__ FtrkState st;
   __shared__ double red[FTRK_WARPS][6];
   const int ch = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
-  const FtrkChanDev c = a.chan[ch];
-  const uint8_t *rec = a.iq + c.rec_off;
   const int L = a.code_len;
-  // caCode = [caCode($) caCode caCode(1)]  (tracking.sci:171-175)
-  for (int i = tid; i < L + 2; i += NT) {
-    const int k = (i == 0) ? L - 1 : (i == L + 1 ? 0 : i - 1);
-    code[i] = (double)a.chips[c.code_row * 1024 + k];
-  }
   // loop state that only lane 0 needs
+  gnssb200_softtrack_state *sp = a.state + ch;
   double oldCodeNco = 0.0, oldCodeError = 0.0, oldCarrNco = 0.0, oldCarrError = 0.0;
-  double I1 = 0.001, Q1 = 0.001;
-  const double carrFreqBasis = c.acquired_freq;
+  double I1 = 0.0, Q1 = 0.0, carrFreqBasis = 0.0;
+  int sv = 0, done = 0, status = 0;
+  bool live = false;  // thread 0: the state is not final (RECORD_END and MS_DONE are; such a channel is left as it is)
   if (tid == 0) {
-    st.codeFreq = a.code_freq_basis;
-    st.remCodePhase = 0.0;
-    st.carrFreq = c.acquired_freq;
-    st.remCarrPhase = 0.0;
-    st.pos = c.start;
-    st.stop = 0;
-    const double step = st.codeFreq / a.fs;
-    st.blksize = (int)ceil(((double)L - st.remCodePhase) / step);
-    if (st.pos < 0 || st.pos + st.blksize > a.n_samples) st.stop = 1;
+    status = sp->status;
+    live = status <= GNSSB200_SOFTTRACK_RUNNING;
+    st.run = 0;
+    if (live) {
+      oldCodeNco = sp->oldCodeNco;
+      oldCodeError = sp->oldCodeError;
+      oldCarrNco = sp->oldCarrNco;
+      oldCarrError = sp->oldCarrError;
+      I1 = sp->I1;
+      Q1 = sp->Q1;
+      carrFreqBasis = sp->carrFreqBasis;
+      sv = sp->sv;
+      done = sp->ms_done;
+      const int record = sp->record;
+      st.codeFreq = sp->codeFreq;
+      st.remCodePhase = sp->remCodePhase;
+      st.carrFreq = sp->carrFreq;
+      st.remCarrPhase = sp->remCarrPhase;
+      st.pos = sp->pos;
+      st.code_row = a.glonass ? 0 : sv;
+      st.rec = a.win + (size_t)record * a.win_stride;
+      const double step = st.codeFreq / a.fs;
+      st.blksize = (int)ceil(((double)L - st.remCodePhase) / step);
+      if (record < 0 || record >= a.n_records)
+        status = GNSSB200_SOFTTRACK_BAD_RECORD;
+      else if (!a.glonass && (sv < 1 || sv > 32))
+        status = GNSSB200_SOFTTRACK_BAD_SV;
+      else
+        status = ftrk_next(a, st.pos, st.blksize, done, &st.run);
+    }
   }
   __syncthreads();
+  if (st.run) {
+    // caCode = [caCode($) caCode caCode(1)]  (tracking.sci:171-175)
+    for (int i = tid; i < L + 2; i += NT) {
+      const int k = (i == 0) ? L - 1 : (i == L + 1 ? 0 : i - 1);
+      code[i] = (double)a.chips[st.code_row * 1024 + k];
+    }
+    __syncthreads();
+  }
+  const uint8_t *rec = st.rec;
   double *out = a.out + (size_t)ch * a.ms * 13;
-  int done = 0;
-  for (int it = 0; it < a.ms; it++) {
-    if (st.stop) break;
+  while (st.run) {
     const double codeFreq = st.codeFreq, rem = st.remCodePhase, carrFreq = st.carrFreq, remCarr = st.remCarrPhase;
-    const long long pos = st.pos;
+    const long long pos = st.pos, wpos = pos - a.win_first;
     const int blksize = st.blksize;
     const double step = codeFreq / a.fs;            // codePhaseStep
     const double w = (carrFreq * 2.0) * M_PI;       // (carrFreq * 2.0 * %pi)
@@ -128,7 +159,7 @@ __global__ void __launch_bounds__(NT) softtrack_kernel(const FtrkArgs a) {
       if (v < blksize) sincos(__dadd_rn(__dmul_rn(w, __ddiv_rn((double)v, a.fs)), remCarr), &sn, &cs);
       for (int j = v; j < blksize; j += FTRK_LANES) {
         double I, Q;
-        ftrk_sample<FMT>(rec, pos + j, I, Q);
+        ftrk_sample<FMT>(rec, wpos + j, I, Q);
         // carrsig .* rawSignal, carrsig = exp(%i*trigarg); qBaseband = real, iBaseband = imag
         const double qb = __dsub_rn(__dmul_rn(cs, I), __dmul_rn(sn, Q));
         const double ib = __dadd_rn(__dmul_rn(cs, Q), __dmul_rn(sn, I));
@@ -189,11 +220,11 @@ __global__ void __launch_bounds__(NT) softtrack_kernel(const FtrkArgs a) {
       double newCodeFreq;
       if (a.glonass)
         newCodeFreq = a.code_freq_basis - codeNco +
-                      (newCarrFreq - (a.IF + a.IF_step * c.sv)) / ((a.zero_channel + c.sv * a.IF_step) / a.code_freq_basis);
+                      (newCarrFreq - (a.IF + a.IF_step * sv)) / ((a.zero_channel + sv * a.IF_step) / a.code_freq_basis);
       else
         newCodeFreq = a.code_freq_basis - codeNco + ((newCarrFreq - a.IF) / 1540);
       const long long newPos = pos + blksize;
-      double *o = out + (size_t)it * 13;
+      double *o = out + (size_t)done * 13;
       o[0] = I_E; o[1] = I_P; o[2] = I_L; o[3] = Q_E; o[4] = Q_P; o[5] = Q_L;
       o[6] = newCarrFreq; o[7] = newCodeFreq; o[8] = codeError; o[9] = codeNco; o[10] = carrError; o[11] = carrNco;
       o[12] = (double)newPos - newRem * (a.fs / 1000) / (double)L;   // absoluteSample (:380-384)
@@ -204,12 +235,29 @@ __global__ void __launch_bounds__(NT) softtrack_kernel(const FtrkArgs a) {
       st.pos = newPos;
       const double nstep = newCodeFreq / a.fs;
       st.blksize = (int)ceil(((double)L - newRem) / nstep);
-      if (newPos + st.blksize > a.n_samples) st.stop = 1;
+      done++;
+      status = ftrk_next(a, newPos, st.blksize, done, &st.run);
     }
-    done = it + 1;
     __syncthreads();
   }
-  if (tid == 0) a.ms_done[ch] = done;
+  if (tid == 0) {  // the state after the last period run, also at a pause
+    if (live) {
+      sp->codeFreq = st.codeFreq;
+      sp->remCodePhase = st.remCodePhase;
+      sp->carrFreq = st.carrFreq;
+      sp->remCarrPhase = st.remCarrPhase;
+      sp->oldCodeNco = oldCodeNco;
+      sp->oldCodeError = oldCodeError;
+      sp->oldCarrNco = oldCarrNco;
+      sp->oldCarrError = oldCarrError;
+      sp->I1 = I1;
+      sp->Q1 = Q1;
+      sp->pos = st.pos;
+      sp->ms_done = done;
+      sp->status = status;
+    }
+    if (a.ms_done) a.ms_done[ch] = sp->ms_done;
+  }
 }
 
 template <int NT>
@@ -255,40 +303,10 @@ static int ftrk_auto_width(gnssb200_handle *h, int fmt, int n_ch, int *nt_out) {
   return 0;
 }
 
-// The tracking of n_ch channels spread over records d_iq + rec*stride; chan_record NULL: every channel in record 0.
-// Arguments are validated by the callers.  Synchronous on cuda_stream.
-static int softtrack_run(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq, size_t stride, int fmt,
-                         int64_t n_samples, const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
-                         double *d_out, int32_t *d_ms_done, void *cuda_stream, int nt) {
-  CUDA_TRY(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)cuda_stream;
-  const int8_t *d_chips = nullptr;
-  if (int rc = chip_table(h, &d_chips)) return rc;
-  const bool glo = cfg->system == GNSSB200_SYS_GLONASS;
-  std::vector<FtrkChanDev> hc(n_ch);
-  for (int i = 0; i < n_ch; i++) {
-    hc[i].sv = chans[i].sv;
-    hc[i].code_row = glo ? 0 : chans[i].sv;
-    hc[i].acquired_freq = chans[i].acquired_freq;
-    hc[i].start = cfg->skip_samples + (int64_t)(chans[i].code_phase - 1);
-    hc[i].rec_off = chan_record ? (long long)((size_t)chan_record[i] * stride) : 0;
-  }
-  FtrkChanDev *d_ch = nullptr;
-  CUDA_TRY(cudaMalloc(&d_ch, sizeof(FtrkChanDev) * n_ch));
-  cudaError_t e = cudaMemcpyAsync(d_ch, hc.data(), sizeof(FtrkChanDev) * n_ch, cudaMemcpyHostToDevice, st);
-  if (e != cudaSuccess) {
-    cudaFree(d_ch);
-    CUDA_TRY(e);
-  }
-  FtrkArgs a;
-  a.iq = (const uint8_t *)d_iq;
-  a.n_samples = n_samples;
-  a.chips = d_chips;
-  a.chan = d_ch;
-  a.out = d_out;
-  a.ms_done = d_ms_done;
+static FtrkArgs ftrk_args(const gnssb200_softtrack_cfg *cfg) {
+  FtrkArgs a = {};
   a.ms = cfg->ms_to_process;
-  a.glonass = glo ? 1 : 0;
+  a.glonass = cfg->system == GNSSB200_SYS_GLONASS ? 1 : 0;
   a.code_len = cfg->code_length;
   a.fs = cfg->samp_freq;
   a.IF = cfg->IF;
@@ -306,22 +324,96 @@ static int softtrack_run(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, 
     a.k2 = 1.414 * p;
     a.k3 = T * (cfg->fll_noise_bandwidth / 0.25);
   }
-  e = cudaEventRecord(h->ev0, st);
-  if (e == cudaSuccess) {
-    if (nt == 128)
-      ftrk_launch_nt<128>(fmt, n_ch, st, a);
-    else if (nt == 256)
-      ftrk_launch_nt<256>(fmt, n_ch, st, a);
-    else
-      ftrk_launch_nt<512>(fmt, n_ch, st, a);
-    e = cudaGetLastError();
+  return a;
+}
+
+// One window of the tracking kernel for the n_ch states of d_state; arguments validated by the callers.  nt: threads
+// per channel, 0 = the handle's width (or the automatic one).  Asynchronous on st.
+static int ftrk_window(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_win, size_t win_stride,
+                       int n_records, int fmt, int64_t win_first, int64_t win_samples, int64_t record_samples,
+                       gnssb200_softtrack_state *d_state, int n_ch, double *d_out, int32_t *d_ms_done, cudaStream_t st,
+                       int nt) {
+  CUDA_TRY(cudaSetDevice(h->device));
+  const int8_t *d_chips = nullptr;
+  if (int rc = chip_table(h, &d_chips)) return rc;
+  if (nt == 0) nt = h->softtrack_width;
+  if (nt == 0)
+    if (int rc = ftrk_auto_width(h, fmt, n_ch, &nt)) return rc;
+  FtrkArgs a = ftrk_args(cfg);
+  a.win = (const uint8_t *)d_win;
+  a.win_stride = win_stride;
+  a.n_records = n_records;
+  a.win_first = win_first;
+  a.win_end = win_first + win_samples;
+  a.record_samples = record_samples;
+  a.chips = d_chips;
+  a.state = d_state;
+  a.out = d_out;
+  a.ms_done = d_ms_done;
+  if (nt == 128)
+    ftrk_launch_nt<128>(fmt, n_ch, st, a);
+  else if (nt == 256)
+    ftrk_launch_nt<256>(fmt, n_ch, st, a);
+  else
+    ftrk_launch_nt<512>(fmt, n_ch, st, a);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return 0;
+}
+
+static int ftrk_bad(int rc, const char *what) {
+  gnssb200_set_error(rc, what, __FILE__, __LINE__);
+  return rc;
+}
+
+extern "C" int gnssb200_softtrack_init(const gnssb200_softtrack_cfg *cfg, const gnssb200_softtrack_chan *chans,
+                                       const int32_t *chan_record, int n_records, int n_ch, gnssb200_softtrack_state *states) {
+  if (!cfg || !chans || !states || n_ch <= 0 || n_records < 1 || cfg->ms_to_process <= 0 ||
+      (cfg->code_length != 511 && cfg->code_length != 1023))
+    return ftrk_bad(-20, "gnssb200_softtrack_init: bad arguments");
+  if (cfg->system != GNSSB200_SYS_GLONASS)
+    for (int i = 0; i < n_ch; i++)
+      if (chans[i].sv < 1 || chans[i].sv > 32) return ftrk_bad(-21, "gnssb200_softtrack_init: GPS PRN must be 1..32");
+  if (chan_record)
+    for (int i = 0; i < n_ch; i++)
+      if (chan_record[i] < 0 || chan_record[i] >= n_records) return ftrk_bad(-24, "gnssb200_softtrack_init: chan_record out of range");
+  for (int i = 0; i < n_ch; i++) {  // tracking.sci:226-250: the loop state before period 1
+    gnssb200_softtrack_state s = {};
+    s.codeFreq = cfg->code_freq;
+    s.carrFreq = chans[i].acquired_freq;
+    s.I1 = 0.001;
+    s.Q1 = 0.001;
+    s.carrFreqBasis = chans[i].acquired_freq;
+    s.pos = cfg->skip_samples + (int64_t)(chans[i].code_phase - 1);
+    s.sv = chans[i].sv;
+    s.record = chan_record ? chan_record[i] : 0;
+    s.status = GNSSB200_SOFTTRACK_RUNNING;
+    states[i] = s;
   }
-  if (e == cudaSuccess) e = cudaEventRecord(h->ev1, st);
-  if (e == cudaSuccess) {
-    h->launches++;
-    e = cudaStreamSynchronize(st);  // hc / d_ch lifetimes
-  }
-  cudaFree(d_ch);
+  return 0;
+}
+
+// The one-shot tracking of n_ch channels spread over records d_iq + rec*stride (chan_record NULL: every channel in
+// record 0): init and one window that covers the whole record.  Arguments are validated by the callers.  Synchronous
+// on cuda_stream.
+static int softtrack_run(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq, size_t stride,
+                         int n_records, int fmt, int64_t n_samples, const gnssb200_softtrack_chan *chans,
+                         const int32_t *chan_record, int n_ch, double *d_out, int32_t *d_ms_done, void *cuda_stream, int nt) {
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  std::vector<gnssb200_softtrack_state> hs(n_ch);
+  if (int rc = gnssb200_softtrack_init(cfg, chans, chan_record, n_records, n_ch, hs.data())) return rc;
+  gnssb200_softtrack_state *d_state = nullptr;
+  CUDA_TRY(cudaMalloc(&d_state, sizeof(gnssb200_softtrack_state) * n_ch));
+  int rc = 0;
+  cudaError_t e = cudaMemcpyAsync(d_state, hs.data(), sizeof(gnssb200_softtrack_state) * n_ch, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaEventRecord(h->ev0, st);
+  if (e == cudaSuccess)
+    rc = ftrk_window(h, cfg, d_iq, stride, n_records, fmt, 0, n_samples, n_samples, d_state, n_ch, d_out, d_ms_done, st, nt);
+  if (e == cudaSuccess && !rc) e = cudaEventRecord(h->ev1, st);
+  if (e == cudaSuccess && !rc) e = cudaStreamSynchronize(st);  // hs / d_state lifetimes
+  cudaFree(d_state);
+  if (rc) return rc;
   CUDA_TRY(e);
   return 0;
 }
@@ -340,47 +432,194 @@ extern "C" int gnssb200_softtrack(gnssb200_handle *h, const gnssb200_softtrack_c
         gnssb200_set_error(-21, "gnssb200_softtrack: GPS PRN must be 1..32", __FILE__, __LINE__);
         return -21;
       }
-  return softtrack_run(h, cfg, d_iq, 0, GNSSB200_FMT_INT8_IQ, n_samples, chans, nullptr, n_ch, d_out, d_ms_done, cuda_stream,
-                       FTRK_LANES);
+  return softtrack_run(h, cfg, d_iq, 0, 1, GNSSB200_FMT_INT8_IQ, n_samples, chans, nullptr, n_ch, d_out, d_ms_done,
+                       cuda_stream, FTRK_LANES);
+}
+
+static size_t ftrk_bytes(int fmt, int64_t n) { return fmt == GNSSB200_FMT_INT8_IQ ? (size_t)n * 2 : ((size_t)n + 1) / 2; }
+
+// The argument checks of gnssb200_softtrack_batch and gnssb200_softtrack_batch_host (d_iq / h_iq, d_out / h_out, ...)
+static int ftrk_check_batch(const char *fn, gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *iq,
+                            size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
+                            const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch, const double *out,
+                            const int32_t *ms_done) {
+  char msg[160];
+  if (!h || !cfg || !iq || !chans || !chan_record || n_ch <= 0 || !out || !ms_done || cfg->ms_to_process <= 0 ||
+      (cfg->code_length != 511 && cfg->code_length != 1023) || n_samples < 0) {
+    snprintf(msg, sizeof msg, "%s: bad arguments", fn);
+    return ftrk_bad(-20, msg);
+  }
+  if (cfg->system != GNSSB200_SYS_GLONASS)
+    for (int i = 0; i < n_ch; i++)
+      if (chans[i].sv < 1 || chans[i].sv > 32) {
+        snprintf(msg, sizeof msg, "%s: GPS PRN must be 1..32", fn);
+        return ftrk_bad(-21, msg);
+      }
+  if (fmt != GNSSB200_FMT_INT8_IQ && fmt != GNSSB200_FMT_PACKED2) {
+    snprintf(msg, sizeof msg, "%s: fmt must be INT8_IQ or PACKED2", fn);
+    return ftrk_bad(-22, msg);
+  }
+  if (n_records < 1 || (record_stride_bytes != 0 && record_stride_bytes < ftrk_bytes(fmt, n_samples))) {
+    snprintf(msg, sizeof msg, "%s: n_records < 1, or a record stride shorter than n_samples in fmt", fn);
+    return ftrk_bad(-23, msg);
+  }
+  for (int i = 0; i < n_ch; i++)
+    if (chan_record[i] < 0 || chan_record[i] >= n_records) {
+      snprintf(msg, sizeof msg, "%s: chan_record out of range", fn);
+      return ftrk_bad(-24, msg);
+    }
+  return 0;
 }
 
 extern "C" int gnssb200_softtrack_batch(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq,
                                         size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
                                         const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
                                         double *d_out, int32_t *d_ms_done, void *cuda_stream) {
-  if (!h || !cfg || !d_iq || !chans || !chan_record || n_ch <= 0 || !d_out || !d_ms_done || cfg->ms_to_process <= 0 ||
-      (cfg->code_length != 511 && cfg->code_length != 1023) || n_samples < 0) {
-    gnssb200_set_error(-20, "gnssb200_softtrack_batch: bad arguments", __FILE__, __LINE__);
-    return -20;
-  }
-  if (cfg->system != GNSSB200_SYS_GLONASS)
-    for (int i = 0; i < n_ch; i++)
-      if (chans[i].sv < 1 || chans[i].sv > 32) {
-        gnssb200_set_error(-21, "gnssb200_softtrack_batch: GPS PRN must be 1..32", __FILE__, __LINE__);
-        return -21;
-      }
-  if (fmt != GNSSB200_FMT_INT8_IQ && fmt != GNSSB200_FMT_PACKED2) {
-    gnssb200_set_error(-22, "gnssb200_softtrack_batch: fmt must be INT8_IQ or PACKED2", __FILE__, __LINE__);
-    return -22;
-  }
-  const size_t rec_bytes = fmt == GNSSB200_FMT_INT8_IQ ? (size_t)n_samples * 2 : ((size_t)n_samples + 1) / 2;
-  if (n_records < 1 || (record_stride_bytes != 0 && record_stride_bytes < rec_bytes)) {
-    gnssb200_set_error(-23, "gnssb200_softtrack_batch: n_records < 1, or a record stride shorter than n_samples in fmt",
-                       __FILE__, __LINE__);
-    return -23;
-  }
-  for (int i = 0; i < n_ch; i++)
-    if (chan_record[i] < 0 || chan_record[i] >= n_records) {
-      gnssb200_set_error(-24, "gnssb200_softtrack_batch: chan_record out of range", __FILE__, __LINE__);
-      return -24;
-    }
-  int nt = h->softtrack_width;
-  if (nt == 0) {
+  if (int rc = ftrk_check_batch("gnssb200_softtrack_batch", h, cfg, d_iq, record_stride_bytes, n_records, fmt, n_samples,
+                                chans, chan_record, n_ch, d_out, d_ms_done))
+    return rc;
+  return softtrack_run(h, cfg, d_iq, record_stride_bytes, n_records, fmt, n_samples, chans, chan_record, n_ch, d_out,
+                       d_ms_done, cuda_stream, 0);
+}
+
+extern "C" int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_win,
+                                         size_t win_stride_bytes, int n_records, int fmt, int64_t win_first,
+                                         int64_t win_samples, int64_t record_samples, gnssb200_softtrack_state *d_state,
+                                         int n_ch, double *d_out, void *cuda_stream) {
+  if (!h || !cfg || !d_win || !d_state || !d_out || n_ch <= 0 || n_records < 1 || win_first < 0 || win_samples < 0 ||
+      cfg->ms_to_process <= 0 || (cfg->code_length != 511 && cfg->code_length != 1023))
+    return ftrk_bad(-20, "gnssb200_softtrack_resume: bad arguments");
+  if (fmt != GNSSB200_FMT_INT8_IQ && fmt != GNSSB200_FMT_PACKED2)
+    return ftrk_bad(-22, "gnssb200_softtrack_resume: fmt must be INT8_IQ or PACKED2");
+  if (fmt == GNSSB200_FMT_PACKED2 && (win_first & 1))
+    return ftrk_bad(-22, "gnssb200_softtrack_resume: a packed window must start on an even sample");
+  if (win_stride_bytes != 0 && win_stride_bytes < ftrk_bytes(fmt, win_samples))
+    return ftrk_bad(-23, "gnssb200_softtrack_resume: a window stride shorter than win_samples in fmt");
+  if (!h->d_chips) {  // the handle's chip table is built by a synchronous upload, which a stream capture cannot hold
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     CUDA_TRY(cudaSetDevice(h->device));
-    if (int rc = ftrk_auto_width(h, fmt, n_ch, &nt)) return rc;
+    CUDA_TRY(cudaStreamIsCapturing((cudaStream_t)cuda_stream, &cap));
+    if (cap != cudaStreamCaptureStatusNone)
+      return ftrk_bad(-27, "gnssb200_softtrack_resume: capture needs one float-tracking call on the handle before it");
   }
-  return softtrack_run(h, cfg, d_iq, record_stride_bytes, fmt, n_samples, chans, chan_record, n_ch, d_out, d_ms_done,
-                       cuda_stream, nt);
+  return ftrk_window(h, cfg, d_win, win_stride_bytes, n_records, fmt, win_first, win_samples, record_samples, d_state, n_ch,
+                     d_out, nullptr, (cudaStream_t)cuda_stream, 0);
+}
+
+// Automatic window of gnssb200_softtrack_batch_host: 2^20 samples (65.5 ms at 16 Msps), fewer if a staging buffer would
+// pass 512 MiB.  Measured on a B200 with 64 records x 8 channels (DESIGN §4.3): 2^20 samples was the fastest of 2^18,
+// 2^20 and 2^22 for int8 (128 MiB buffers) and of 2^20, 2^22 and 2^24 for packed (32 MiB), 1.03-1.12x the larger of the
+// kernel time and the copy time.  Longer windows leave a longer first copy and last kernel without overlap.
+#define FTRK_AUTO_WINDOW_SAMPLES (1LL << 20)
+#define FTRK_MAX_STAGE_BYTES ((size_t)512 << 20)
+
+extern "C" int gnssb200_softtrack_batch_host(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *h_iq,
+                                             size_t stride, int n_records, int fmt, int64_t n_samples,
+                                             const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
+                                             double *h_out, int32_t *h_ms_done, int64_t window_samples) {
+  if (int rc = ftrk_check_batch("gnssb200_softtrack_batch_host", h, cfg, h_iq, stride, n_records, fmt, n_samples, chans,
+                                chan_record, n_ch, h_out, h_ms_done))
+    return rc;
+  // nominal code period P; windows overlap by 2P (even for packed input, so every window starts on an even sample)
+  const double period = ceil((double)cfg->code_length * cfg->samp_freq / cfg->code_freq);
+  const long long P = period >= 1.0 && period < 1e9 ? (long long)period : 0;
+  if (P == 0 || window_samples < 0 || (window_samples > 0 && window_samples < 4 * P))
+    return ftrk_bad(-26, "gnssb200_softtrack_batch_host: window_samples must be 0 or at least four code periods");
+  const bool packed = fmt == GNSSB200_FMT_PACKED2;
+  const long long O = packed ? (2 * P + 1) & ~1LL : 2 * P;
+  const int rows_copied = stride ? n_records : 1;  // stride 0: one record, read n_records times
+  long long W = window_samples;
+  if (W == 0) {
+    const long long rec_bytes = (long long)(FTRK_MAX_STAGE_BYTES / rows_copied);
+    const long long cap = packed ? 2 * rec_bytes : rec_bytes / 2;
+    W = FTRK_AUTO_WINDOW_SAMPLES < cap ? FTRK_AUTO_WINDOW_SAMPLES : cap;
+    if (W < 4 * P) W = 4 * P;
+  }
+  if (W > n_samples) W = n_samples;  // one window holds the whole record: staging memory follows the input
+  long long A = W - O;  // advance from one window to the next
+  if (packed) A &= ~1LL;
+  const size_t wbytes = ftrk_bytes(fmt, W);
+  const size_t dpitch = (wbytes + 255) & ~(size_t)255;
+  CUDA_TRY(cudaSetDevice(h->device));
+  int rc = 0;
+  auto fail = [&](cudaError_t e, int line) {
+    gnssb200_set_error((int)e, cudaGetErrorString(e), __FILE__, line);
+    rc = (int)e;
+  };
+#define TRY_(x)                                       \
+  do {                                                \
+    cudaError_t e_ = (x);                             \
+    if (e_ != cudaSuccess && !rc) fail(e_, __LINE__); \
+  } while (0)
+  // the handle's staging streams, events and buffers, shared with gnssb200_track_run_host (both synchronise)
+  if (!h->s_copy) {
+    TRY_(cudaStreamCreateWithFlags(&h->s_copy, cudaStreamNonBlocking));
+    TRY_(cudaStreamCreateWithFlags(&h->s_comp, cudaStreamNonBlocking));
+    TRY_(cudaStreamCreateWithFlags(&h->s_back, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; i++) {
+      TRY_(cudaEventCreateWithFlags(&h->ev_copied[i], cudaEventDisableTiming));
+      TRY_(cudaEventCreateWithFlags(&h->ev_used[i], cudaEventDisableTiming));
+    }
+  }
+  const size_t stage_need = dpitch * rows_copied + 256;
+  if (!rc && stage_need > h->stage_cap) {
+    for (int i = 0; i < 2; i++) {
+      cudaFree(h->stage[i]);
+      h->stage[i] = nullptr;
+      TRY_(cudaMalloc(&h->stage[i], stage_need));
+    }
+    h->stage_cap = rc ? 0 : stage_need;
+  }
+  std::vector<gnssb200_softtrack_state> hs(n_ch);
+  if (!rc) rc = gnssb200_softtrack_init(cfg, chans, chan_record, n_records, n_ch, hs.data());
+  gnssb200_softtrack_state *d_state = nullptr;
+  double *d_out = nullptr;
+  const size_t ch_rows = (size_t)cfg->ms_to_process * GNSSB200_SOFTTRACK_FIELDS;
+  if (!rc) TRY_(cudaMalloc(&d_state, sizeof(gnssb200_softtrack_state) * n_ch));
+  if (!rc) TRY_(cudaMalloc(&d_out, sizeof(double) * ch_rows * n_ch));
+  cudaStream_t s_copy = h->s_copy, s_comp = h->s_comp;
+  if (!rc)
+    TRY_(cudaMemcpyAsync(d_state, hs.data(), sizeof(gnssb200_softtrack_state) * n_ch, cudaMemcpyHostToDevice, s_comp));
+  if (!rc) TRY_(cudaEventRecord(h->ev0, s_comp));
+  for (long long k = 0, first = 0; !rc; k++, first += A) {
+    const long long len = n_samples - first < W ? n_samples - first : W;
+    const int buf = (int)(k & 1);
+    if (k >= 2) TRY_(cudaStreamWaitEvent(s_copy, h->ev_used[buf], 0));  // the kernel of window k-2 is done with it
+    const size_t lbytes = ftrk_bytes(fmt, len);
+    if (lbytes)
+      TRY_(cudaMemcpy2DAsync(h->stage[buf], dpitch, (const uint8_t *)h_iq + (packed ? first / 2 : 2 * first),
+                             stride ? stride : lbytes, lbytes, rows_copied, cudaMemcpyHostToDevice, s_copy));
+    TRY_(cudaEventRecord(h->ev_copied[buf], s_copy));
+    TRY_(cudaStreamWaitEvent(s_comp, h->ev_copied[buf], 0));
+    if (!rc)
+      rc = ftrk_window(h, cfg, h->stage[buf], stride ? dpitch : 0, n_records, fmt, first, len, n_samples, d_state, n_ch,
+                       d_out, nullptr, s_comp, 0);
+    TRY_(cudaEventRecord(h->ev_used[buf], s_comp));
+    if (first + W >= n_samples) break;
+  }
+  if (!rc) TRY_(cudaEventRecord(h->ev1, s_comp));
+  if (!rc)
+    TRY_(cudaMemcpyAsync(hs.data(), d_state, sizeof(gnssb200_softtrack_state) * n_ch, cudaMemcpyDeviceToHost, s_comp));
+  if (s_comp) TRY_(cudaStreamSynchronize(s_comp));
+  if (s_copy) TRY_(cudaStreamSynchronize(s_copy));
+  int stopped = 0;
+  if (!rc) {
+    for (int i = 0; i < n_ch && !rc; i++) {
+      if (hs[i].ms_done > 0)
+        TRY_(cudaMemcpyAsync(h_out + ch_rows * i, d_out + ch_rows * i, sizeof(double) * GNSSB200_SOFTTRACK_FIELDS * hs[i].ms_done,
+                             cudaMemcpyDeviceToHost, s_comp));
+      // the last window reaches the record end, so every channel ends RECORD_END or MS_DONE unless a block was
+      // longer than the overlap; a pos before sample 0 stops the one-shot call as well
+      if (hs[i].status == GNSSB200_SOFTTRACK_BEHIND && hs[i].pos >= 0) stopped++;
+    }
+    TRY_(cudaStreamSynchronize(s_comp));
+    if (!rc)
+      for (int i = 0; i < n_ch; i++) h_ms_done[i] = hs[i].ms_done;
+  }
+  cudaFree(d_state);
+  cudaFree(d_out);
+#undef TRY_
+  return rc ? rc : stopped;
 }
 
 extern "C" int gnssb200_set_softtrack_width(gnssb200_handle *h, int threads) {

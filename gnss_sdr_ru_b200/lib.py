@@ -106,6 +106,12 @@ def lib() -> C.CDLL:
         L.gnssb200_softtrack_batch.argtypes = [vp, P(abi.SoftTrackCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, vp, vp, C.c_int,
                                                vp, vp, vp]
         L.gnssb200_set_softtrack_width.argtypes = [vp, C.c_int]
+    if hasattr(L, "gnssb200_softtrack_resume"):
+        L.gnssb200_softtrack_init.argtypes = [P(abi.SoftTrackCfg), vp, vp, C.c_int, C.c_int, vp]
+        L.gnssb200_softtrack_resume.argtypes = [vp, P(abi.SoftTrackCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, i64, i64, vp,
+                                                C.c_int, vp, vp]
+        L.gnssb200_softtrack_batch_host.argtypes = [vp, P(abi.SoftTrackCfg), vp, C.c_size_t, C.c_int, C.c_int, i64, vp, vp,
+                                                    C.c_int, vp, vp, i64]
     _lib = L
     return L
 

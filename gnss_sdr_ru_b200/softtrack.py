@@ -75,6 +75,30 @@ def _track_results(out: np.ndarray, done: np.ndarray, channel: list) -> list:
     return res
 
 
+def _per_record(out: np.ndarray, done: np.ndarray, channels: list) -> list:
+    """One trackResults list per record from the rows and periods of the flat channel list."""
+    res, i = [], 0
+    for chl in channels:
+        res.append(_track_results(out[i : i + len(chl)], done[i : i + len(chl)], chl))
+        i += len(chl)
+    return res
+
+
+def _flat_channels(channels: list, n_records: int):
+    """The channel table and chan_record of one preRun channel list per record, flattened record by record."""
+    if len(channels) != n_records:
+        raise ValueError("channels must hold one channel list per record")
+    flat = [(r, c) for r, chl in enumerate(channels) for c in chl]
+    ch = (abi.SoftTrackChan * len(flat))()
+    rec = (C.c_int32 * len(flat))()
+    for i, (r, c) in enumerate(flat):
+        ch[i].sv = c["FCH"]
+        ch[i].code_phase = c["codePhase"]
+        ch[i].acquired_freq = c["acquiredFreq"]
+        rec[i] = r
+    return ch, rec
+
+
 class SoftTrackingEngine:
     def __init__(self, device: int = 0, handle=None):
         self.L = lib()
@@ -127,18 +151,9 @@ class SoftTrackingEngine:
         """gnssb200_softtrack_batch: record r at d_iq_ptr + r*stride (stride 0: one record n_records times) in fmt
         (FMT_INT8_IQ or FMT_PACKED2).  channels holds one preRun channel list per record; they are tracked as one
         flat list, record by record, into d_out [n_ch][msToProcess][13] and d_ms_done [n_ch].  Synchronous on `stream`."""
-        if len(channels) != n_records:
-            raise ValueError("channels must hold one channel list per record")
-        flat = [(r, c) for r, chl in enumerate(channels) for c in chl]
-        ch = (abi.SoftTrackChan * len(flat))()
-        rec = (C.c_int32 * len(flat))()
-        for i, (r, c) in enumerate(flat):
-            ch[i].sv = c["FCH"]
-            ch[i].code_phase = c["codePhase"]
-            ch[i].acquired_freq = c["acquiredFreq"]
-            rec[i] = r
+        ch, rec = _flat_channels(channels, n_records)
         cfg = settings.to_c()
-        check(self.L.gnssb200_softtrack_batch(self.h, C.byref(cfg), d_iq_ptr, stride, n_records, fmt, n_samples, ch, rec, len(flat),
+        check(self.L.gnssb200_softtrack_batch(self.h, C.byref(cfg), d_iq_ptr, stride, n_records, fmt, n_samples, ch, rec, len(ch),
                                               d_out_ptr, d_ms_done_ptr, stream or None), "gnssb200_softtrack_batch")
 
     def tracking_batch(self, d_iq_ptr: int, stride: int, n_records: int, n_samples: int, channels: list, settings: TrackSettings,
@@ -156,12 +171,53 @@ class SoftTrackingEngine:
         d_done = torch.zeros(n_ch, dtype=torch.int32, device=dev)
         self.tracking_batch_device(d_iq_ptr, stride, n_records, n_samples, channels, settings, d_out.data_ptr(), d_done.data_ptr(),
                                    fmt=fmt, stream=torch.cuda.current_stream().cuda_stream)
-        out, done = d_out.cpu().numpy(), d_done.cpu().numpy()
-        res, i = [], 0
-        for chl in channels:
-            res.append(_track_results(out[i : i + len(chl)], done[i : i + len(chl)], chl))
-            i += len(chl)
-        return res
+        return _per_record(d_out.cpu().numpy(), d_done.cpu().numpy(), channels)
+
+    def init_states(self, channels: list, settings: TrackSettings, n_records: int):
+        """gnssb200_softtrack_init: the state of every channel before its first code period, as a ctypes array of
+        abi.SoftTrackState (host memory).  channels holds one preRun channel list per record, flattened record by record
+        as in tracking_batch_device."""
+        ch, rec = _flat_channels(channels, n_records)
+        states = (abi.SoftTrackState * len(ch))()
+        cfg = settings.to_c()
+        check(self.L.gnssb200_softtrack_init(C.byref(cfg), ch, rec, n_records, len(ch), states), "gnssb200_softtrack_init")
+        return states
+
+    def resume_device(self, d_win_ptr: int, win_stride: int, n_records: int, fmt: int, win_first: int, win_samples: int,
+                      record_samples: int, settings: TrackSettings, d_state_ptr: int, n_ch: int, d_out_ptr: int, stream: int = 0):
+        """gnssb200_softtrack_resume: continue the n_ch device states d_state_ptr through samples [win_first, win_first +
+        win_samples) of every record (record r's window at d_win_ptr + r*win_stride), rows into d_out [n_ch][msToProcess][13].
+        Asynchronous on `stream`."""
+        cfg = settings.to_c()
+        check(self.L.gnssb200_softtrack_resume(self.h, C.byref(cfg), d_win_ptr, win_stride, n_records, fmt, win_first, win_samples,
+                                               record_samples, d_state_ptr, n_ch, d_out_ptr, stream or None),
+              "gnssb200_softtrack_resume")
+
+    def tracking_batch_host(self, h_iq, stride: int, n_records: int, n_samples: int, channels: list, settings: TrackSettings,
+                            fmt: int = abi.FMT_INT8_IQ, window_samples: int = 0) -> list:
+        """tracking_batch on records in host memory (a numpy array or a CPU torch tensor, pinned for copies that overlap
+        the tracking), staged window by window: one list of trackResults dicts per record.  The number of channels
+        stopped because a block was longer than the windows' overlap (normally 0) is left in self.host_stopped."""
+        if hasattr(h_iq, "data_ptr"):
+            if h_iq.is_cuda or not h_iq.is_contiguous():
+                raise ValueError("h_iq must be a contiguous host tensor")
+            ptr = h_iq.data_ptr()
+        else:
+            h_iq = np.ascontiguousarray(h_iq)
+            ptr = h_iq.ctypes.data
+        ch, rec = _flat_channels(channels, n_records)
+        n_ch = len(ch)
+        if n_ch == 0:
+            return [[] for _ in channels]
+        out = np.zeros((n_ch, settings.msToProcess, 13), dtype=np.float64)
+        done = np.zeros(n_ch, dtype=np.int32)
+        cfg = settings.to_c()
+        rc = self.L.gnssb200_softtrack_batch_host(self.h, C.byref(cfg), ptr, stride, n_records, fmt, n_samples, ch, rec, n_ch,
+                                                  out.ctypes.data, done.ctypes.data, window_samples)
+        if rc < 0:
+            check(rc, "gnssb200_softtrack_batch_host")
+        self.host_stopped = rc
+        return _per_record(out, done, channels)
 
     def set_width(self, threads: int):
         """Threads per channel of the batched call: 0 automatic, 128, 256 or 512.  Results do not depend on it."""

@@ -445,10 +445,88 @@ int gnssb200_softtrack_batch(gnssb200_handle *h, const gnssb200_softtrack_cfg *c
                              const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
                              double *d_out, int32_t *d_ms_done, void *cuda_stream);
 
-/* Threads per channel of gnssb200_softtrack_batch: 0 automatic, else 128, 256 or 512.  Results do not depend on it.
- * Automatic: the width whose CTAs finish all channels in the fewest waves, weighted by the measured time of a wave at
- * that width -- 512 while every channel has an SM of its own, narrower beyond that (DESIGN §4.3). */
+/* Threads per channel of gnssb200_softtrack_batch and gnssb200_softtrack_resume: 0 automatic, else 128, 256 or 512.
+ * Results do not depend on it.  Automatic: the width whose CTAs finish all channels in the fewest waves, weighted by
+ * the measured time of a wave at that width -- 512 while every channel has an SM of its own, narrower beyond that
+ * (DESIGN §4.3). */
 int gnssb200_set_softtrack_width(gnssb200_handle *h, int threads);
+
+/* Resumable float tracking.  gnssb200_softtrack_state holds one channel between two code periods: everything the
+ * tracking loop carries from one period to the next.  The block size is not stored; the kernel recomputes it as
+ * (int)ceil((code_length - remCodePhase) / (codeFreq / samp_freq)), the expression of the loop itself, and doubles
+ * round-trip exactly through memory.  So a channel tracked window by window (gnssb200_softtrack_resume), or
+ * checkpointed to the host and continued on another handle, gives rows and ms_done byte-identical to
+ * gnssb200_softtrack_batch on the whole record, at any kernel width. */
+#define GNSSB200_SOFTTRACK_RUNNING     0  /* not finished: paused at a window end (or not started yet) */
+#define GNSSB200_SOFTTRACK_RECORD_END  1  /* the next block passes the record end (pos + blksize > record_samples) */
+#define GNSSB200_SOFTTRACK_MS_DONE     2  /* ms_done reached ms_to_process */
+#define GNSSB200_SOFTTRACK_BEHIND     -1  /* pos < win_first: the next block starts before the window; nothing was read */
+#define GNSSB200_SOFTTRACK_BAD_RECORD -2  /* record outside 0..n_records-1; nothing was read */
+#define GNSSB200_SOFTTRACK_BAD_SV     -3  /* GPS PRN outside 1..32; nothing was read */
+
+typedef struct gnssb200_softtrack_state {
+  double codeFreq, remCodePhase;  /* code NCO */
+  double carrFreq, remCarrPhase;  /* carrier NCO */
+  double oldCodeNco, oldCodeError, oldCarrNco, oldCarrError;  /* loop-filter memory */
+  double I1, Q1;                  /* the FLL's previous prompt sums; 0.001 before period 1 */
+  double carrFreqBasis;           /* channel.acquiredFreq */
+  int64_t pos;                    /* first sample of the next block, in the channel's record */
+  int32_t sv;                     /* PRN (GPS) / FCH (GLONASS) */
+  int32_t record;                 /* record index */
+  int32_t ms_done;                /* rows written so far: the next row is d_out[ch][ms_done] */
+  int32_t status;                 /* GNSSB200_SOFTTRACK_* */
+} gnssb200_softtrack_state;
+
+/* The state every channel has before its first code period: codeFreq = code_freq, carrFreq = carrFreqBasis =
+ * acquired_freq, remainders and loop memory 0, I1 = Q1 = 0.001, pos = skip_samples + code_phase - 1,
+ * record = chan_record[i] (NULL: 0), status RUNNING.  Host code, no device.  Validates as gnssb200_softtrack_batch:
+ * -20 (NULL pointer, n_ch <= 0, n_records < 1, ms_to_process <= 0, code length other than 511 / 1023), -21 (GPS PRN
+ * outside 1..32), -24 (chan_record out of range); states are untouched then. */
+int gnssb200_softtrack_init(const gnssb200_softtrack_cfg *cfg, const gnssb200_softtrack_chan *chans,
+                            const int32_t *chan_record, int n_records, int n_ch, gnssb200_softtrack_state *states);
+
+/* Track the n_ch channels of d_state [n_ch] (device) through one window of samples: samples
+ * [win_first, win_first + win_samples) of every record.  Record r's window starts at d_win + r*win_stride_bytes
+ * (0: every record is the same buffer).  INT8_IQ: sample k at byte 2*(k - win_first).  PACKED2: sample k is nibble
+ * k & 1 of byte (k >> 1) - (win_first >> 1); win_first must be even.
+ * A channel runs code periods while ms_done < ms_to_process, its next block [pos, pos + blksize) lies inside the window
+ * and pos + blksize <= record_samples (the reference's end rule).  A block that runs past the window end pauses the
+ * channel (status RUNNING, state unchanged), and a later window continues it; consecutive windows must overlap by at
+ * least the block length.  record_samples may be any value at or past the window end while the record's true length
+ * is not yet known; the end rule applies from the call that passes the true length.  A channel whose pos lies before
+ * win_first stops as BEHIND, one with a record index out of range as BAD_RECORD: nothing is read or written for them
+ * but the status.  Channels whose status is RECORD_END or MS_DONE are left untouched.  Rows go to
+ * d_out [n_ch][ms_to_process][13], row ms_done of the channel, the layout of gnssb200_softtrack_batch.
+ * Uses the width of gnssb200_set_softtrack_width (or the automatic width); it may change between windows.
+ * Device pointers and scalars only, asynchronous on cuda_stream.  It can be captured in a CUDA graph once the handle
+ * holds its chip table, i.e. after any float-tracking call on the handle (gnssb200_softtrack*, or one resume outside
+ * the capture); under capture without it the call returns -27.  Returns < 0 and launches
+ * nothing for: fmt other than INT8_IQ / PACKED2, packed input with an odd win_first, a non-zero stride shorter than
+ * the window's bytes, n_records < 1, n_ch <= 0, win_first < 0, win_samples < 0, ms_to_process <= 0, a NULL pointer,
+ * a code length other than 511 / 1023. */
+int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_win,
+                              size_t win_stride_bytes, int n_records, int fmt, int64_t win_first, int64_t win_samples,
+                              int64_t record_samples, gnssb200_softtrack_state *d_state, int n_ch, double *d_out,
+                              void *cuda_stream);
+
+/* gnssb200_softtrack_batch on records in host memory: h_iq is a host buffer (record r at h_iq + r*record_stride_bytes,
+ * 0: one record), h_out [n_ch][ms_to_process][13] and h_ms_done [n_ch] are host arrays; only rows [0, ms_done) of a
+ * channel are written.  The records are staged window by window through two device buffers of one window of all
+ * records each (cudaMemcpy2DAsync on a copy stream), the copy of window k+1 under the tracking of window k.
+ * Consecutive windows overlap by two nominal code periods, 2*ceil(code_length*samp_freq/code_freq) samples, so a
+ * channel paused at a window end finds its next block whole in the next window.  Device memory: the two staging
+ * buffers, the rows and the states; the records are never resident whole.  Pinned host memory (cudaHostAlloc /
+ * cudaHostRegister) gives the overlap; pageable memory gives the same results without it.
+ * window_samples: samples per window, 0 automatic (2^20 samples, fewer if one window of all records would pass 512 MiB; DESIGN §4.3); below four
+ * nominal code periods it is invalid; a window longer than the record is cut to the record.  Returns 0, or the number
+ * of channels that ended BEHIND at pos >= 0 -- a block longer than the overlap, or a diverged loop whose block size
+ * turned non-positive and walked pos back before a later window (the one-shot call would run such a channel on towards
+ * sample 0) -- whose rows up to that point are still those of the one-shot call; or < 0 for the invalid arguments of
+ * gnssb200_softtrack_batch and an invalid window_samples (-26), with h_out / h_ms_done untouched.  Synchronous. */
+int gnssb200_softtrack_batch_host(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *h_iq,
+                                  size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
+                                  const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
+                                  double *h_out, int32_t *h_ms_done, int64_t window_samples);
 
 /* ---------------------------------------------------------------------------------------------
  * (2) batched layer -- streaming ingest (SURVEY.md 8f, rank 4): a circular buffer between a sample
