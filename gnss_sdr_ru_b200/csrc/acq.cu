@@ -359,6 +359,12 @@ extern "C" int gnssb200_acq_search_batch(gnssb200_handle *h, const gnssb200_acq_
                        __FILE__, __LINE__);
     return -15;
   }
+  // sample_at reads an int8 I,Q sample as one 2-byte char2 load: the records must start on even addresses
+  if (fmt == GNSSB200_FMT_INT8_IQ && (((uintptr_t)d_iq | record_stride_bytes) & 1)) {
+    gnssb200_set_error(-15, "gnssb200_acq_search_batch: int8 I,Q records need an even d_iq and an even record stride",
+                       __FILE__, __LINE__);
+    return -15;
+  }
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (!h->acq_ws) h->acq_ws = new AcqWorkspace();

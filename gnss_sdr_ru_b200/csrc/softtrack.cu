@@ -366,10 +366,29 @@ static int ftrk_bad(int rc, const char *what) {
   return rc;
 }
 
+// The correlator spacing the kernel can read: 0 <= spc <= 0.5 chip (NaN fails).  The early / prompt / late chips are
+// code[ceil(rem -+ spc + j*step)] of the padded period code[0..L+1] = [caCode($) caCode caCode(1)], for the samples
+// j = 0..blksize-1 of a block.  blksize = ceil((L - rem) / step) puts rem + j*step in [rem, L), and the remainder
+// carried into the next block, rem + blksize*step - L, lies in [0, step), both up to rounding: rem is exactly 0 in
+// period 1 and can be a few 1e-13 below 0 after it.  The early index ceil(rem - spc) >= 0 needs spc < 1 + rem, the
+// late index ceil(t + spc) <= L + 1 (t < L) needs spc <= 1 less the rounding of t.  With rem a little below 0 no bound
+// just under 1 chip is airtight; 0.5 chip each side, the widest conventional spacing (10x the GLONASS default 0.05,
+// 2.5x the GPS one 0.2), leaves half a chip for rounding.  (The reference stops on an index outside the padded code:
+// Scilab raises on index 0 or L + 3.)
+static bool ftrk_spacing_ok(const gnssb200_softtrack_cfg *cfg) {
+  return cfg->dll_correlator_spacing >= 0.0 && cfg->dll_correlator_spacing <= 0.5;
+}
+
+// int8 I,Q samples are read as 2-byte char2 loads, which need an even address: the record base and its stride must be
+// even.  Packed records are read byte by byte and may start anywhere.
+static bool ftrk_aligned(int fmt, const void *base, size_t stride) {
+  return fmt != GNSSB200_FMT_INT8_IQ || !(((uintptr_t)base | stride) & 1);
+}
+
 extern "C" int gnssb200_softtrack_init(const gnssb200_softtrack_cfg *cfg, const gnssb200_softtrack_chan *chans,
                                        const int32_t *chan_record, int n_records, int n_ch, gnssb200_softtrack_state *states) {
   if (!cfg || !chans || !states || n_ch <= 0 || n_records < 1 || cfg->ms_to_process <= 0 ||
-      (cfg->code_length != 511 && cfg->code_length != 1023))
+      (cfg->code_length != 511 && cfg->code_length != 1023) || !ftrk_spacing_ok(cfg))
     return ftrk_bad(-20, "gnssb200_softtrack_init: bad arguments");
   if (cfg->system != GNSSB200_SYS_GLONASS)
     for (int i = 0; i < n_ch; i++)
@@ -422,10 +441,13 @@ extern "C" int gnssb200_softtrack(gnssb200_handle *h, const gnssb200_softtrack_c
                                   const gnssb200_softtrack_chan *chans, int n_ch, double *d_out, int32_t *d_ms_done,
                                   void *cuda_stream) {
   if (!h || !cfg || !d_iq || !chans || n_ch <= 0 || !d_out || !d_ms_done || cfg->ms_to_process <= 0 ||
-      (cfg->code_length != 511 && cfg->code_length != 1023)) {  // the kernel's chip buffer holds one ST or C/A period
+      (cfg->code_length != 511 && cfg->code_length != 1023) ||  // the kernel's chip buffer holds one ST or C/A period
+      !ftrk_spacing_ok(cfg)) {
     gnssb200_set_error(-20, "gnssb200_softtrack: bad arguments", __FILE__, __LINE__);
     return -20;
   }
+  if (!ftrk_aligned(GNSSB200_FMT_INT8_IQ, d_iq, 0))
+    return ftrk_bad(-23, "gnssb200_softtrack: an int8 I,Q record must start on an even byte address");
   if (cfg->system != GNSSB200_SYS_GLONASS)
     for (int i = 0; i < n_ch; i++)
       if (chans[i].sv < 1 || chans[i].sv > 32) {
@@ -445,7 +467,7 @@ static int ftrk_check_batch(const char *fn, gnssb200_handle *h, const gnssb200_s
                             const int32_t *ms_done) {
   char msg[160];
   if (!h || !cfg || !iq || !chans || !chan_record || n_ch <= 0 || !out || !ms_done || cfg->ms_to_process <= 0 ||
-      (cfg->code_length != 511 && cfg->code_length != 1023) || n_samples < 0) {
+      (cfg->code_length != 511 && cfg->code_length != 1023) || !ftrk_spacing_ok(cfg) || n_samples < 0) {
     snprintf(msg, sizeof msg, "%s: bad arguments", fn);
     return ftrk_bad(-20, msg);
   }
@@ -478,6 +500,8 @@ extern "C" int gnssb200_softtrack_batch(gnssb200_handle *h, const gnssb200_softt
   if (int rc = ftrk_check_batch("gnssb200_softtrack_batch", h, cfg, d_iq, record_stride_bytes, n_records, fmt, n_samples,
                                 chans, chan_record, n_ch, d_out, d_ms_done))
     return rc;
+  if (!ftrk_aligned(fmt, d_iq, record_stride_bytes))
+    return ftrk_bad(-23, "gnssb200_softtrack_batch: int8 I,Q records need an even d_iq and an even record stride");
   return softtrack_run(h, cfg, d_iq, record_stride_bytes, n_records, fmt, n_samples, chans, chan_record, n_ch, d_out,
                        d_ms_done, cuda_stream, 0);
 }
@@ -487,7 +511,7 @@ extern "C" int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_soft
                                          int64_t win_samples, int64_t record_samples, gnssb200_softtrack_state *d_state,
                                          int n_ch, double *d_out, void *cuda_stream) {
   if (!h || !cfg || !d_win || !d_state || !d_out || n_ch <= 0 || n_records < 1 || win_first < 0 || win_samples < 0 ||
-      cfg->ms_to_process <= 0 || (cfg->code_length != 511 && cfg->code_length != 1023))
+      cfg->ms_to_process <= 0 || (cfg->code_length != 511 && cfg->code_length != 1023) || !ftrk_spacing_ok(cfg))
     return ftrk_bad(-20, "gnssb200_softtrack_resume: bad arguments");
   if (fmt != GNSSB200_FMT_INT8_IQ && fmt != GNSSB200_FMT_PACKED2)
     return ftrk_bad(-22, "gnssb200_softtrack_resume: fmt must be INT8_IQ or PACKED2");
@@ -495,6 +519,8 @@ extern "C" int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_soft
     return ftrk_bad(-22, "gnssb200_softtrack_resume: a packed window must start on an even sample");
   if (win_stride_bytes != 0 && win_stride_bytes < ftrk_bytes(fmt, win_samples))
     return ftrk_bad(-23, "gnssb200_softtrack_resume: a window stride shorter than win_samples in fmt");
+  if (!ftrk_aligned(fmt, d_win, win_stride_bytes))
+    return ftrk_bad(-23, "gnssb200_softtrack_resume: int8 I,Q windows need an even d_win and an even window stride");
   if (!h->d_chips) {  // the handle's chip table is built by a synchronous upload, which a stream capture cannot hold
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     CUDA_TRY(cudaSetDevice(h->device));

@@ -337,7 +337,8 @@ int gnssb200_acq_num_bins(const gnssb200_acq_cfg *cfg);
 /* Samples the record must hold: n_noncoh<=1 -> 2*coh_ms ms, else n_noncoh*coh_ms ms. */
 int64_t gnssb200_acq_samples_needed(const gnssb200_acq_cfg *cfg);
 
-/* Grid search on a device-resident int8 I,Q record (fmt INT8_IQ or PACKED2).
+/* Grid search on a device-resident int8 I,Q record (fmt INT8_IQ or PACKED2).  An INT8_IQ record must start on an
+ * even byte address (its samples are read as 2-byte loads); a PACKED2 record may start anywhere.
  *   d_rows   device buffer [n_sv * n_bins] of rows; only this partition's rows are written
  *            (others keep peak = -1).  Multi-GPU callers all-gather this table (NCCL) and then call
  *            gnssb200_acq_finalize on the merged table.
@@ -348,6 +349,7 @@ int gnssb200_acq_search(gnssb200_handle *h, const gnssb200_acq_cfg *cfg, const v
 /* The same search over R = n_records records with the same settings in one call (gnssb200_acq_search is the case
  * R = 1).  Record r starts at d_iq + r*record_stride_bytes (0 = every record is the same buffer), e.g. the stream
  * buffer that gnssb200_track_run then consumes; a non-zero stride must cover the bytes n_samples takes in fmt.
+ * INT8_IQ: d_iq and the stride must be even (-15 otherwise, as for a short stride).
  *   d_rows   device [R][n_sv][n_bins]: record r's table is laid out exactly like gnssb200_acq_search's, with the same
  *            partition rule (part_index / part_count).
  * The handle's workspace holds the base spectra of all R records: R * n_cls * K * 128 KB, n_cls = the number of
@@ -409,7 +411,9 @@ typedef struct gnssb200_softtrack_cfg {
   double IF_step;                 /* settings.L1_IF_step (GLONASS) */
   double glonass_zero_channel;    /* settings.GLONASS_zero_channel 1602e6 */
   double code_freq;               /* settings.codeFreqBasis */
-  double dll_damping_ratio, dll_noise_bandwidth, dll_correlator_spacing;
+  double dll_damping_ratio, dll_noise_bandwidth;
+  double dll_correlator_spacing;  /* settings.dllCorrelatorSpacing, chips: 0 <= spacing <= 0.5 (NaN is invalid), so
+                                   * the early and late chips stay inside the period padded by one chip each side */
   double pll_noise_bandwidth, fll_noise_bandwidth;
   int64_t skip_samples;           /* settings.skipNumberOfBytes in complex samples */
   int32_t ms_to_process;          /* settings.msToProcess */
@@ -424,8 +428,10 @@ typedef struct gnssb200_softtrack_chan {   /* one entry of the `channel` struct 
 
 #define GNSSB200_SOFTTRACK_FIELDS 13 /* I_E I_P I_L Q_E Q_P Q_L carrFreq codeFreq dllDiscr dllDiscrFilt pllDiscr pllDiscrFilt absoluteSample */
 
-/* d_iq: device int8 I,Q record (the whole file); d_out: device double [n_ch][ms_to_process][13];
- * d_ms_done: device int32 [n_ch] = code periods actually processed (fewer if the record ends).
+/* d_iq: device int8 I,Q record (the whole file) at an even byte address; d_out: device double
+ * [n_ch][ms_to_process][13]; d_ms_done: device int32 [n_ch] = code periods actually processed (fewer if the record
+ * ends).  Returns < 0 and writes nothing for -20 (NULL pointer, n_ch <= 0, ms_to_process <= 0, code length other than
+ * 511 / 1023, dll_correlator_spacing outside 0..0.5 or NaN), -21 (GPS PRN outside 1..32), -23 (odd d_iq).
  * Synchronous on cuda_stream. */
 int gnssb200_softtrack(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq, int64_t n_samples,
                        const gnssb200_softtrack_chan *chans, int n_ch, double *d_out, int32_t *d_ms_done,
@@ -437,9 +443,11 @@ int gnssb200_softtrack(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, co
  * it starts at cfg->skip_samples + chans[i].code_phase - 1 of that record and stops at that record's end.
  * d_out [n_ch][ms_to_process][13] and d_ms_done [n_ch] are laid out exactly as gnssb200_softtrack's, and each
  * channel's values are bit-identical to gnssb200_softtrack on its record alone (after unpacking, for PACKED2),
- * whatever kernel width runs.  Returns < 0 and writes nothing to d_out / d_ms_done when an argument is invalid
- * (n_records < 1, a chan_record out of range, another fmt, a stride that does not cover a record, a GPS PRN outside
- * 1..32, a code length other than 511 / 1023, n_ch <= 0).  Synchronous on cuda_stream. */
+ * whatever kernel width runs.  Returns < 0 and writes nothing to d_out / d_ms_done when an argument is invalid:
+ * -20 (NULL pointer, n_ch <= 0, ms_to_process <= 0, a code length other than 511 / 1023, dll_correlator_spacing
+ * outside 0..0.5 or NaN), -21 (a GPS PRN outside 1..32), -22 (another fmt), -23 (n_records < 1, a stride that does not
+ * cover a record, or for INT8_IQ an odd d_iq or an odd stride), -24 (a chan_record out of range).
+ * Synchronous on cuda_stream. */
 int gnssb200_softtrack_batch(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_iq,
                              size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
                              const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,
@@ -480,8 +488,9 @@ typedef struct gnssb200_softtrack_state {
 /* The state every channel has before its first code period: codeFreq = code_freq, carrFreq = carrFreqBasis =
  * acquired_freq, remainders and loop memory 0, I1 = Q1 = 0.001, pos = skip_samples + code_phase - 1,
  * record = chan_record[i] (NULL: 0), status RUNNING.  Host code, no device.  Validates as gnssb200_softtrack_batch:
- * -20 (NULL pointer, n_ch <= 0, n_records < 1, ms_to_process <= 0, code length other than 511 / 1023), -21 (GPS PRN
- * outside 1..32), -24 (chan_record out of range); states are untouched then. */
+ * -20 (NULL pointer, n_ch <= 0, n_records < 1, ms_to_process <= 0, code length other than 511 / 1023,
+ * dll_correlator_spacing outside 0..0.5 or NaN), -21 (GPS PRN outside 1..32), -24 (chan_record out of range); states
+ * are untouched then. */
 int gnssb200_softtrack_init(const gnssb200_softtrack_cfg *cfg, const gnssb200_softtrack_chan *chans,
                             const int32_t *chan_record, int n_records, int n_ch, gnssb200_softtrack_state *states);
 
@@ -501,9 +510,10 @@ int gnssb200_softtrack_init(const gnssb200_softtrack_cfg *cfg, const gnssb200_so
  * Device pointers and scalars only, asynchronous on cuda_stream.  It can be captured in a CUDA graph once the handle
  * holds its chip table, i.e. after any float-tracking call on the handle (gnssb200_softtrack*, or one resume outside
  * the capture); under capture without it the call returns -27.  Returns < 0 and launches
- * nothing for: fmt other than INT8_IQ / PACKED2, packed input with an odd win_first, a non-zero stride shorter than
- * the window's bytes, n_records < 1, n_ch <= 0, win_first < 0, win_samples < 0, ms_to_process <= 0, a NULL pointer,
- * a code length other than 511 / 1023. */
+ * nothing for: -22 (fmt other than INT8_IQ / PACKED2, packed input with an odd win_first), -23 (a non-zero stride
+ * shorter than the window's bytes; INT8_IQ with an odd d_win or an odd stride), -20 (n_records < 1, n_ch <= 0,
+ * win_first < 0, win_samples < 0, ms_to_process <= 0, a NULL pointer, a code length other than 511 / 1023,
+ * dll_correlator_spacing outside 0..0.5 or NaN). */
 int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *d_win,
                               size_t win_stride_bytes, int n_records, int fmt, int64_t win_first, int64_t win_samples,
                               int64_t record_samples, gnssb200_softtrack_state *d_state, int n_ch, double *d_out,
@@ -522,7 +532,8 @@ int gnssb200_softtrack_resume(gnssb200_handle *h, const gnssb200_softtrack_cfg *
  * of channels that ended BEHIND at pos >= 0 -- a block longer than the overlap, or a diverged loop whose block size
  * turned non-positive and walked pos back before a later window (the one-shot call would run such a channel on towards
  * sample 0) -- whose rows up to that point are still those of the one-shot call; or < 0 for the invalid arguments of
- * gnssb200_softtrack_batch and an invalid window_samples (-26), with h_out / h_ms_done untouched.  Synchronous. */
+ * gnssb200_softtrack_batch (h_iq and the stride may be odd: windows are staged into aligned device buffers) and an
+ * invalid window_samples (-26), with h_out / h_ms_done untouched.  Synchronous. */
 int gnssb200_softtrack_batch_host(gnssb200_handle *h, const gnssb200_softtrack_cfg *cfg, const void *h_iq,
                                   size_t record_stride_bytes, int n_records, int fmt, int64_t n_samples,
                                   const gnssb200_softtrack_chan *chans, const int32_t *chan_record, int n_ch,

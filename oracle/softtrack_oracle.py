@@ -162,15 +162,26 @@ def replay(rec: dict, channel: dict, s: TrackSettings):
     return {f: np.array(v) for f, v in out.items()}
 
 
-def tracking(iq_int8: np.ndarray, channel: dict, s: TrackSettings):
+def _chips(caCode: np.ndarray, t: np.ndarray, what: str) -> np.ndarray:
+    """caCode(ceil(tcode)+1) (1-based) as a 0-based lookup; an index outside the padded code raises, as in Scilab."""
+    idx = np.ceil(t).astype(np.int64)
+    if idx.size and (idx.min() < 0 or idx.max() > caCode.size - 1):
+        raise IndexError(f"{what} code index {int(idx.min())}..{int(idx.max())} outside 0..{caCode.size - 1} "
+                         "(Scilab: invalid index)")
+    return caCode[idx]
+
+
+def tracking(iq_int8: np.ndarray, channel: dict, s: TrackSettings, left_pad: float | None = None):
     """One channel of tracking.sci.  iq_int8: interleaved I,Q record (the whole file).  Returns a dict of
-    arrays of length msToProcess (shorter if the record ends)."""
+    arrays of length msToProcess (shorter if the record ends).  A code index outside the padded code raises
+    IndexError, where Scilab stops with an invalid index (a correlator spacing of a chip or more in period 1).
+    left_pad replaces the value of caCode($) at the front of the padded code (mutation checks; None: the reference)."""
     x = np.asarray(iq_int8, dtype=np.int8)
     sig_all = x[0::2].astype(np.float64) + 1j * x[1::2].astype(np.float64)
     fs = s.samplingFreq
     L = s.codeLength
     code = (ca_code(channel["FCH"]) if s.system == "gps" else st_code()).astype(np.float64)
-    caCode = np.concatenate([code[-1:], code, code[:1]])
+    caCode = np.concatenate([code[-1:] if left_pad is None else [float(left_pad)], code, code[:1]])
     earlyLateSpc = s.dllCorrelatorSpacing
     lf = LoopFilters(s, channel)
     pos = s.skipNumberOfSamples + (channel["codePhase"] - 1)
@@ -192,9 +203,9 @@ def tracking(iq_int8: np.ndarray, channel: dict, s: TrackSettings):
         tE = (remCodePhase - earlyLateSpc) + j * codePhaseStep
         tL = (remCodePhase + earlyLateSpc) + j * codePhaseStep
         tP = remCodePhase + j * codePhaseStep
-        earlyCode = caCode[np.ceil(tE).astype(np.int64)]   # Scilab: caCode(ceil(tcode)+1), 1-based
-        lateCode = caCode[np.ceil(tL).astype(np.int64)]
-        promptCode = caCode[np.ceil(tP).astype(np.int64)]
+        earlyCode = _chips(caCode, tE, "early")   # Scilab: caCode(ceil(tcode)+1), 1-based
+        lateCode = _chips(caCode, tL, "late")
+        promptCode = _chips(caCode, tP, "prompt")
         remCodePhase = (tP[blksize - 1] + codePhaseStep) - L
         time = np.arange(blksize + 1, dtype=np.float64) / fs
         trigarg = ((carrFreq * 2.0 * np.pi) * time) + remCarrPhase
